@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — GCN training edges/sec on synthetic graphs (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1..5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1..5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workloads (BASELINE.json `configs`, --config; the default, 2, is the one the metric is quoted on):
@@ -23,6 +23,10 @@ DRAM traffic ncu measured for that (config, N) when profiles/sg_traffic.json has
 `--impl reference` time the CPU oracle (OpenMP, all host cores, thread count set explicitly) on a bounded sample
 of the same workload — ROC ships no CPU kernels (SURVEY §8c/d).  For N > 1 a `parity_check` (outside the timed
 region) trains a bounded graph on the N-rank engine and on a 1-rank engine and compares logits / loss / dW.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step handed back (see dump_outputs) as
+DIR/<name>.npy.  Graph, features, labels, mask and initial weights all come from fixed seeds, so two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import importlib.util
@@ -44,6 +48,7 @@ LR, WD = 0.01, 0.0001          # example_run.sh: -lr 0.01 -decay 0.0001
 BASE_SCALE = 22
 BASE_PAIRS = 1 << 25
 CPU_SAMPLE_SCALE = 19          # cpu_baseline / reference arm: same generator, 1/8 of the vertices
+DUMP_ROWS = 1 << 16            # --dump-outputs: logits rows written (at most 47 classes: 12 MB)
 
 CONFIGS = {
     1: dict(kind="gcn", layers=[16, 16, 5], graph="uniform", scaling="strong",
@@ -218,7 +223,7 @@ def run_reference(args, rank, world):
         return
     cfg = CONFIGS[args.config]
     layers = cfg["layers"] if cfg["kind"] == "gcn" else CONFIGS[2]["layers"]
-    steps = max(5, min(args.steps, 10))
+    steps = args.steps
     warm = max(1, min(args.warmup, 2))
     rate, best, ms, info = cpu_epoch_rate(steps, warm, layers)
     info["value"] = rate
@@ -244,6 +249,26 @@ def build_model(m, cfg):
     if c["kind"] == "gcn":
         return build_gcn(m, c["layers"], DROPOUT, lr=LR, weight_decay=WD)
     return build_sage_mean(m, c["layers"], DROPOUT, lr=LR, weight_decay=WD)
+
+
+def dump_outputs(outdir, m, hnd, perf, row_left):
+    """--dump-outputs: the logits of the last timed forward pass (rank 0's rows; a fixed, seeded sample of
+    DUMP_ROWS of them when there are more, with their global ids in logits_rows), its loss metrics (PerfMetrics
+    order), and every weight and weight gradient after its update — fp32 / fp64, about 20 MB at most."""
+    from roc_b200._lib import PerfMetrics
+    os.makedirs(outdir, exist_ok=True)
+    logits = m.get_tensor(hnd["logits"])
+    rows = np.arange(logits.shape[0])
+    if rows.shape[0] > DUMP_ROWS:
+        rows = np.sort(np.random.RandomState(0).choice(rows.shape[0], DUMP_ROWS, replace=False))
+    out = {"logits": logits[rows], "logits_rows": (row_left + rows).astype(np.float64),
+           "metrics": np.array([perf[k] for k, _ in PerfMetrics._fields_], dtype=np.float64)}
+    for p in range(m.num_parameters()):
+        out["weight%d" % p] = m.get_parameter(p)
+        out["weight%d_grad" % p] = m.get_parameter(p, "grad")
+    for name, a in out.items():
+        np.save(os.path.join(outdir, name + ".npy"), a)
+    log("[bench] wrote %d arrays (%.1f MB) to %s" % (len(out), sum(a.nbytes for a in out.values()) / 1e6, outdir))
 
 
 def parity_check(rank, local_rank, world, dist, dev):
@@ -416,6 +441,8 @@ def run_ours(args, rank, local_rank, world):
     clocks = sampler.stop() if rank == 0 else None
     perf = m.metrics()
     value = e * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:    # before the end-to-end arm trains further
+        dump_outputs(args.dump_outputs, m, hnd, perf, rl)
 
     # ---- end-to-end arm: host buffers in, metrics out, every step
     def e2e_step():
@@ -554,7 +581,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer leg (profiling runs)")
     ap.add_argument("--no-parity", action="store_true", help="skip the N-rank vs 1-rank parity check (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -1,3 +1,4 @@
+import importlib.util
 import os
 import sys
 
@@ -17,11 +18,20 @@ def pytest_configure(config):
 GOLDEN = os.path.join(ROOT, "tests", "golden", "ref_golden.npz")
 
 
+def golden_module(name):
+    """tests/golden/<name>.py: the scripts that minted the golden files also define their seeded inputs."""
+    spec = importlib.util.spec_from_file_location(name, os.path.join(ROOT, "tests", "golden", name + ".py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
 @pytest.fixture(scope="session")
 def golden():
-    if not os.path.exists(GOLDEN):
-        pytest.skip("tests/golden/ref_golden.npz not minted yet (tests/golden/make_golden.py on a GPU box)")
-    return np.load(GOLDEN)
+    """The reference's outputs (tests/golden/ref_golden.npz) together with the seeded inputs they came from."""
+    g = dict(np.load(GOLDEN))
+    g.update(golden_module("make_golden").inputs())
+    return g
 
 
 def rel_close(got, want, rtol=1e-4, atol_scale=1e-5, what=""):

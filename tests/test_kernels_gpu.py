@@ -9,7 +9,7 @@ import numpy as np
 import pytest
 import torch
 
-from conftest import rel_close
+from conftest import golden_module, rel_close
 from oracle import oracle, ref
 from roc_b200 import _lib, datasets
 from roc_b200 import kernels as K
@@ -461,11 +461,12 @@ def test_kernels_vs_reference_golden(golden):
     n = re.shape[0]
     d_re, d_col = to_dev(re, col)
     plan = K.SgPlan(0, n - 1, 0, d_re, d_col)
+    rows = g["A_rows"]
     for h in (16, 41, 64):
         x = torch.from_numpy(g["A_sg_in_%d" % h]).to(DEV)
-        rel_close(plan.forward(x, out=torch.empty((n, h), device=DEV)).cpu().numpy(), g["A_sg_out_%d" % h],
+        rel_close(plan.forward(x, out=torch.empty((n, h), device=DEV)).cpu().numpy()[rows], g["A_sg_out_%d" % h],
                   what="vs aggre_coop_kernel H=%d" % h)
-        assert np.array_equal(K.indegree_norm(0, n - 1, 0, d_re, x).cpu().numpy(), g["A_norm_out_%d" % h])
+        assert np.array_equal(K.indegree_norm(0, n - 1, 0, d_re, x).cpu().numpy()[rows], g["A_norm_out_%d" % h])
     rp, es, _ = K.build_csr(0, n - 1, 0, d_re, d_col)
     assert np.array_equal(es.cpu().numpy().astype(np.uint32), g["A_edgestructs"])
     x, w, dy = (torch.from_numpy(g[k]).to(DEV) for k in ("lin_X", "lin_W", "lin_dY"))
@@ -487,38 +488,40 @@ def test_kernels_vs_reference_golden(golden):
     rel_close(dw.cpu().numpy(), g["adam_w_out"], rtol=1e-6, what="vs adam_update")
 
 
-@pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libroc_ref.so not built (no /root/reference here)")
-def test_side_by_side_with_reference_kernel():
-    re_t, col_t = datasets.rmat_graph(14, 150000, seed=8)
-    row_end, col = re_t.numpy().astype(np.uint64), col_t.numpy().astype(np.uint32)
+def test_side_by_side_with_reference_kernel(golden):
+    """The planned kernel on an R-MAT scale-14 graph with hub rows, at every hidden width of the variants, against
+    the reference's aggre_coop_kernel: its outputs minted on a B200 (tests/golden/make_golden.py, graph C), and
+    live on the whole output when oracle/_ref is there."""
+    mg = golden_module("make_golden")
+    row_end, col = mg.side_by_side_graph()
+    assert mg.col_checksum(col) == int(golden["C_col_crc32"][0]), "the R-MAT generator no longer makes graph C"
     n = row_end.shape[0]
     d_re, d_col = to_dev(row_end, col)
-    rp, es = ref.edge_structs(d_col, d_re, 0, 0)
     plan = K.SgPlan(0, n - 1, 0, d_re, d_col)
-    for h in (16, 64, 128, 256):
-        x = torch.rand((n, h), device=DEV) - 0.5
-        want = ref.scatter_gather(0, n - 1, 0, rp, es, x)
+    if ref.available():
+        rp, es = ref.edge_structs(d_col, d_re, 0, 0)
+    for h in mg.SIDE_BY_SIDE_H:
+        x = torch.from_numpy(mg.side_by_side_input(n, h)).to(DEV)
         got = plan.forward(x)
         torch.cuda.synchronize()
-        rel_close(got.cpu().numpy(), want.cpu().numpy(), what="vs live aggre_coop_kernel H=%d" % h)
+        rel_close(got.cpu().numpy()[golden["C_rows"]], golden["C_sg_out_%d" % h],
+                  what="vs golden aggre_coop_kernel H=%d" % h)
+        if ref.available():
+            want = ref.scatter_gather(0, n - 1, 0, rp, es, x)
+            rel_close(got.cpu().numpy(), want.cpu().numpy(), what="vs live aggre_coop_kernel H=%d" % h)
 
 
 # ---------------------------------------- tcgen05 Linear vs the reference library at the headline shapes ---
 LIN_GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_golden_linear.npz")
 
 
-def _lin_inputs(n, i, o):
-    r = np.random.RandomState(1000 * i + o)        # tests/golden/make_golden_linear.py
-    return (r.rand(n, i).astype(np.float32) * 2 - 1, r.rand(o, i).astype(np.float32) * 2 - 1,
-            r.rand(n, o).astype(np.float32) * 2 - 1)
-
-
 @pytest.mark.parametrize("n,i,o", [(1000, 602, 64), (1000, 64, 41)])
 def test_tcgen05_linear_meets_the_reference_cublas(n, i, o):
     """BASELINE.json configs[1]'s two Linear shapes, fed row-padded so the tcgen05 / TMEM kernels run (asserted
     through roc_last_gemm_path) — against outputs of the REFERENCE's cublasSgemm calls (linear_kernel.cu:76-80,
-    220-231) minted on a B200 by tests/golden/make_golden_linear.py, and live against oracle/_ref when it is there."""
-    X, W, dY = _lin_inputs(n, i, o)
+    220-231) minted on a B200 by tests/golden/make_golden_linear.py at a sample of rows, and live on the whole
+    outputs against oracle/_ref when it is there."""
+    X, W, dY = golden_module("make_golden_linear").inputs(n, i, o)
     xp = K.padded(n, i, DEV, fill=torch.from_numpy(X).to(DEV))
     w = torch.from_numpy(W).to(DEV)
     gyp = K.padded(n, o, DEV, fill=torch.from_numpy(dY).to(DEV))
@@ -530,23 +533,20 @@ def test_tcgen05_linear_meets_the_reference_cublas(n, i, o):
     assert _lib.lib.roc_last_gemm_path(1) == 1 and _lib.lib.roc_last_gemm_path(2) == 1, "dW / dX not on tcgen05"
     torch.cuda.synchronize()
     k = "%dx%dx%d" % (n, i, o)
-    wants = []
-    if os.path.exists(LIN_GOLDEN):
-        g = np.load(LIN_GOLDEN)
-        wants.append(("golden", g["Y_" + k], g["dW_" + k], g["dX_" + k]))
+    g = np.load(LIN_GOLDEN)
+    rows, wrows = g["rows_" + k], g["wrows_" + k]
+    rel_close(y.cpu().numpy()[rows], g["Y_" + k], what="Y vs golden")
+    rel_close(dw.cpu().numpy()[wrows], g["dW_" + k], what="dW vs golden")
+    rel_close(dx.cpu().numpy()[rows], g["dX_" + k], what="dX vs golden")
     if ref.available():
         xd, gyd = torch.from_numpy(X).to(DEV), torch.from_numpy(dY).to(DEV)
         ry = ref.linear_fwd(xd, w, relu=False)
         rw, rx = torch.zeros_like(w), torch.zeros_like(xd)
         ref.linear_bwd(xd, w, ry, gyd.clone(), rw, rx, relu=False)
         torch.cuda.synchronize()
-        wants.append(("live reference", ry.cpu().numpy(), rw.cpu().numpy(), rx.cpu().numpy()))
-    if not wants:
-        pytest.skip("neither tests/golden/ref_golden_linear.npz nor oracle/_ref is present")
-    for name, wy, wdw, wdx in wants:
-        rel_close(y.cpu().numpy(), wy, what="Y vs %s" % name)
-        rel_close(dw.cpu().numpy(), wdw, what="dW vs %s" % name)
-        rel_close(dx.cpu().numpy(), wdx, what="dX vs %s" % name)
+        rel_close(y.cpu().numpy(), ry.cpu().numpy(), what="Y vs live reference")
+        rel_close(dw.cpu().numpy(), rw.cpu().numpy(), what="dW vs live reference")
+        rel_close(dx.cpu().numpy(), rx.cpu().numpy(), what="dX vs live reference")
 
 
 def test_unpadded_linear_reports_the_simt_fallback():

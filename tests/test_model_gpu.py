@@ -137,7 +137,7 @@ def test_glorot_weights_match_reference_curand(golden):
     assert np.array_equal(got["w0"][1], golden["glorot_846930886_16x5"])
     big = make_case(n=64, pairs=100, layers=(602, 64, 3))
     got = run_product(*big, (602, 64, 3), 0.0, 1, True)
-    assert np.array_equal(got["w0"][0], golden["glorot_1804289383_602x64"])
+    assert np.array_equal(got["w0"][0][golden["glorot_602x64_rows"]], golden["glorot_1804289383_602x64"])
 
 
 def test_file_loaders_and_driver(tmp_path):

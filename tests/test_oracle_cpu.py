@@ -181,10 +181,11 @@ def test_oracle_vs_reference_kernels(golden):
     g = golden
     re, col = g["A_row_end"], g["A_col"]
     n = re.shape[0]
+    rows = g["A_rows"]
     for h in (16, 41, 64):
-        rel_close(oracle.scatter_gather(0, n - 1, 0, re, col, g["A_sg_in_%d" % h]), g["A_sg_out_%d" % h],
+        rel_close(oracle.scatter_gather(0, n - 1, 0, re, col, g["A_sg_in_%d" % h])[rows], g["A_sg_out_%d" % h],
                   what="aggre_coop_kernel H=%d" % h)
-        got = oracle.indegree_norm(0, n - 1, 0, re, g["A_sg_in_%d" % h])
+        got = oracle.indegree_norm(0, n - 1, 0, re, g["A_sg_in_%d" % h])[rows]
         assert np.array_equal(got, g["A_norm_out_%d" % h]), "norm_coop_kernel must match bit for bit"
     rp, es = oracle.build_csr(0, n - 1, 0, re, col)
     assert np.array_equal(rp, g["A_rowptrs"]) and np.array_equal(es, g["A_edgestructs"])
@@ -192,14 +193,16 @@ def test_oracle_vs_reference_kernels(golden):
     assert np.array_equal(vb, g["A_vb2"]) and np.array_equal(eb, g["A_eb2"])
     for c in range(2):
         rl, rr, cl, cr = int(vb[c, 0]), int(vb[c, 1]), int(eb[c, 0]), int(eb[c, 1])
-        rel_close(oracle.scatter_gather(rl, rr, cl, re[rl:rr + 1], col[cl:cr + 1], g["A_sg_in_16"]),
+        prow = g["A_p%d_rows" % c]
+        rel_close(oracle.scatter_gather(rl, rr, cl, re[rl:rr + 1], col[cl:cr + 1], g["A_sg_in_16"])[prow],
                   g["A_p%d_sg_out_16" % c], what="partition %d sg" % c)
         _, es_c = oracle.build_csr(rl, rr, cl, re[rl:rr + 1], col[cl:cr + 1])
         assert np.array_equal(es_c, g["A_p%d_edgestructs" % c])
-        assert np.array_equal(oracle.indegree_norm(rl, rr, cl, re[rl:rr + 1], g["A_sg_in_16"][rl:rr + 1]),
+        assert np.array_equal(oracle.indegree_norm(rl, rr, cl, re[rl:rr + 1], g["A_sg_in_16"][rl:rr + 1])[prow],
                               g["A_p%d_norm_out_16" % c])
     re, col = g["B_row_end"], g["B_col"]
-    rel_close(oracle.scatter_gather(0, re.shape[0] - 1, 0, re, col, g["B_sg_in_32"]), g["B_sg_out_32"], what="rmat sg")
+    rel_close(oracle.scatter_gather(0, re.shape[0] - 1, 0, re, col, g["B_sg_in_32"])[g["B_rows"]], g["B_sg_out_32"],
+              what="rmat sg")
 
 
 def test_oracle_vs_reference_library_ops(golden):
@@ -272,16 +275,13 @@ def test_oracle_linear_against_reference_cublas_at_headline_shapes(n, i, o):
     (linear_kernel.cu:76-80, 220-231) at BASELINE.json configs[1]'s two shapes — minted on a B200 by
     tests/golden/make_golden_linear.py (the small 200 x 33 . 9 case lives in ref_golden.npz)."""
     import os
-    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_golden_linear.npz")
-    if not os.path.exists(path):
-        pytest.skip("tests/golden/ref_golden_linear.npz not minted")
-    g = np.load(path)
-    r = np.random.RandomState(1000 * i + o)            # the generator's inputs
-    X, W, dY = (r.rand(n, i).astype(np.float32) * 2 - 1, r.rand(o, i).astype(np.float32) * 2 - 1,
-                r.rand(n, o).astype(np.float32) * 2 - 1)
+    from conftest import golden_module
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_golden_linear.npz"))
+    X, W, dY = golden_module("make_golden_linear").inputs(n, i, o)
     k = "%dx%dx%d" % (n, i, o)
-    rel_close(oracle.linear_fwd(X, W), g["Y_" + k], what="oracle Y vs reference cublasSgemm")
+    rows, wrows = g["rows_" + k], g["wrows_" + k]
+    rel_close(oracle.linear_fwd(X, W)[rows], g["Y_" + k], what="oracle Y vs reference cublasSgemm")
     dw = np.zeros_like(W)
     dx = oracle.linear_bwd(X, W, None, dY.copy(), dw, need_dx=True)
-    rel_close(dw, g["dW_" + k], what="oracle dW vs reference cublasSgemm")
-    rel_close(dx, g["dX_" + k], what="oracle dX vs reference cublasSgemm")
+    rel_close(dw[wrows], g["dW_" + k], what="oracle dW vs reference cublasSgemm")
+    rel_close(dx[rows], g["dX_" + k], what="oracle dX vs reference cublasSgemm")
