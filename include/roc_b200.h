@@ -61,10 +61,19 @@ typedef void*    roc_stream_t; /* cudaStream_t */
 
 /* epilogue fused into the ScatterGather store (what the model applies right
  * after it, gnn.cc:83-85): NORM = the following indegree_norm, RELU = the relu
- * after that.  Applied in that order. */
+ * after that.  Applied in that order.  MEAN divides the row's sum by (float)deg
+ * (one IEEE division; degree-0 rows stay 0): the AVG aggregator.  It combines with
+ * RELU (MEAN first); MEAN | NORM is rejected. */
 #define ROC_SG_EPI_NONE 0
 #define ROC_SG_EPI_NORM 1
 #define ROC_SG_EPI_RELU 2
+#define ROC_SG_EPI_MEAN 4
+
+/* AggrType of gnn.h:75-80 (the values of roc_gnn.h's enum) */
+#define ROC_AGGR_AVG 0
+#define ROC_AGGR_MAX 1
+#define ROC_AGGR_MIN 2
+#define ROC_AGGR_SUM 3
 
 /* PerfMetrics, softmax_kernel.cu:35-39 (same field order) */
 typedef struct {
@@ -151,6 +160,31 @@ int roc_sg_backward(roc_vid_t rowLeft, roc_vid_t rowRight, roc_eid_t colLeft, in
                     const roc_eid_t* rowEnd, const roc_vid_t* colSrc,
                     const float* outGrad, float* inGrad, roc_stream_t stream);
 
+/* MAX / MIN aggregation (aggr = ROC_AGGR_MAX | ROC_AGGR_MIN) over the plan's rows:
+ *   out[v-rowLeft][h] = max / min over e in in(v) of in[col(e)][h]
+ *   arg[v-rowLeft][h] = colGlobal[e] of the winning edge
+ * The winner is the FIRST edge in CSR order among equal values; a NaN candidate replaces a non-NaN best (the
+ * first NaN wins, like torch.amax); +-inf are ordinary values.  Degree-0 rows: out = 0, arg = 0xFFFFFFFF.
+ * colGlobal (u32, parallel to the plan's colSrc) is the canonical global source id of each edge, so that arg
+ * means the same on every partition; NULL = the plan's own colSrc (single partition).  arg == NULL skips the arg
+ * stores (no backward follows).  Same chunk schedule as roc_sg_forward_planned, no atomics, bit-reproducible.
+ * Always the register kernel (ROC_SG_VARIANT does not apply); widths past 1024 floats run in column blocks,
+ * unaligned leading dimensions take a scalar path.  `arg` needs ldArg >= H u32 per row. */
+int roc_sg_aggr_forward(const roc_sg_plan* plan, int aggr, int H, const float* in, int64_t ldIn,
+                        const roc_vid_t* colGlobal, float* out, int64_t ldOut, uint32_t* arg,
+                        int64_t ldArg, roc_stream_t stream);
+/* Backward of MAX / MIN, as a gather over the same plan (no atomics, no reverse exchange):
+ *   inGrad[u-rowLeft][h] = sum over e in in(u) of (arg[col(e)][h] == u ? outGrad[col(e)][h] : skipped)
+ * outGrad and arg are indexed like the forward's input (col ids: global, or local + halo rows); the sum runs in
+ * the plan's per-row order.  Exact only where SUM's backward is (quirk Q1): the in-edge CSR must be symmetric and
+ * free of duplicate edges, so that in(u) lists every v whose in-edges contain u.  Ties send the whole gradient
+ * to the recorded winner. */
+int roc_sg_arg_backward(const roc_sg_plan* plan, int H, const float* outGrad, int64_t ldG, const uint32_t* arg,
+                        int64_t ldArg, roc_vid_t rowLeft, float* inGrad, int64_t ldIn, roc_stream_t stream);
+/* Pre-size the u32 carry slots roc_sg_aggr_forward uses for rows cut at chunk boundaries (like
+ * roc_sg_plan_reserve for the float ones, which it also reserves), for widths up to maxH. */
+int roc_sg_plan_reserve_arg(roc_sg_plan* plan, int maxH);
+
 /* ----------------------------------------------------------------- halo --- */
 
 /* Boundary-node structures of one partition (multi-GPU).  The reference hands every
@@ -211,6 +245,11 @@ int roc_indegree_norm(roc_vid_t rowLeft, roc_vid_t rowRight, roc_eid_t colLeft, 
                       const roc_eid_t* rowEnd, const float* in, int64_t ldIn,
                       float* out, int64_t ldOut, const float* also_relu_mask_of,
                       roc_stream_t stream);
+/* out[n][h] = in[n][h] / (float)deg(n), IEEE division (row-uniform reciprocal form, bit-identical to `/`);
+ * degree-0 rows give 0.  The AVG aggregator's backward scaling (D^-1 dOut). */
+int roc_indegree_div(roc_vid_t rowLeft, roc_vid_t rowRight, roc_eid_t colLeft, int H,
+                     const roc_eid_t* rowEnd, const float* in, int64_t ldIn, float* out,
+                     int64_t ldOut, roc_stream_t stream);
 
 /* Replaces cudnnActivationForward/Backward, activation_kernel.cu:64-66, 128-132.
  * bwd: dX (+)= dY * f'(.) evaluated from the OUTPUT y; accumulate != 0 adds

@@ -181,7 +181,12 @@ public:
   Model(const Graph& _graph, Context _ctx, Runtime* _runtime);
   Tensor add(const Tensor& _input1, const Tensor& _input2);
   Tensor dropout(const Tensor& _input, float rate, int seed = 0);
-  Tensor scatter_gather(const Tensor& _input);
+  /* aggr: the neighbourhood reduction (gnn.h:75-80).  SUM is the reference's ScatterGather; AVG divides each
+   * row's sum by its in-degree; MAX / MIN take the per-column extreme (first edge in CSR order wins ties, NaN
+   * wins over numbers), with gradients routed to the recorded winner.  The backward of every aggregator assumes
+   * a symmetric in-edge CSR without duplicate edges, like SUM's (quirk Q1).  Only SUM ops take part in the
+   * epilogue fusions. */
+  Tensor scatter_gather(const Tensor& _input, AggrType aggr = AGGR_SUM);
   void softmax_cross_entropy(const Tensor& logits, const Tensor& labels, const Tensor& mask);
   Tensor indegree_norm(const Tensor& _input);
   Tensor linear(const Tensor& _input, int outDim, ActiMode activation, Initializer* initializer = NULL);
@@ -244,10 +249,13 @@ public:
 
 class ScatterGather : public GnnOp {  /* gnn.h:225-242, scattergather.cc */
 public:
-  ScatterGather(const Model& model, const Tensor& input);
+  ScatterGather(const Model& model, const Tensor& input, AggrType aggr = AGGR_SUM);
   virtual void init(const Model& model);
   virtual void forward(const Model& model);
   virtual void backward(const Model& model);
+  AggrType aggr;
+  int scratch;       /* AVG: region of the backward's D^-1 dOut rows (+ halo rows); -1 otherwise */
+  int argRegion;     /* MAX / MIN: region of the u32 winner ids [rows (+ halo)][ld] the backward reads; -1 otherwise */
   int epilogue;      /* ROC_SG_EPI_* the forward store applies (set by Model::init fusion) */
   int bwdEpilogue;   /* same for the backward launch */
   int fwdOut, bwdOut;/* region the fused forward / backward writes (-1: own output / input grad) */

@@ -40,6 +40,8 @@ int roc_host_dropout(roc_host* h, int t, float rate, int seed);
 int roc_host_linear(roc_host* h, int t, int outDim, int activation);
 int roc_host_indegree_norm(roc_host* h, int t);
 int roc_host_scatter_gather(roc_host* h, int t);
+/* Model::scatter_gather(t, aggr) with aggr = ROC_AGGR_AVG | _MAX | _MIN | _SUM (roc_b200.h). */
+int roc_host_scatter_gather_aggr(roc_host* h, int t, int aggr);
 int roc_host_relu(roc_host* h, int t);
 int roc_host_sigmoid(roc_host* h, int t);
 int roc_host_add(roc_host* h, int a, int b);
@@ -80,6 +82,10 @@ int roc_host_metrics(roc_host* h, roc_perf_metrics* out);
  * stream around each roc_sg_forward_planned): enable, run steps, read {H, ms}. */
 int roc_host_profile_sg(roc_host* h, int on);
 int roc_host_profile_sg_read(roc_host* h, int maxEntries, int* H, float* ms);
+/* Test hook: the winner ids ([rows][hidden] u32, global vertex ids, 0xFFFFFFFF for degree-0 rows) of the
+ * MAX / MIN scatter_gather whose output is tensor `outTensor`, for this partition's own rows, as the latest
+ * training-mode forward left them.  -1 if that tensor is not the output of such an op. */
+int roc_host_sg_arg(roc_host* h, int outTensor, uint32_t* host);
 
 #ifdef __cplusplus
 }

@@ -14,7 +14,10 @@ ROC_OK = 0
 ROC_ERR_INVALID, ROC_ERR_UNSUPPORTED, ROC_ERR_NOMEM, ROC_ERR_NO_DEVICE, ROC_ERR_IO = -1, -2, -3, -4, -5
 AC_MODE_NONE, AC_MODE_RELU, AC_MODE_SIGMOID = 0, 1, 2
 MASK_TRAIN, MASK_VAL, MASK_TEST, MASK_NONE = 0, 1, 2, 3
-SG_EPI_NONE, SG_EPI_NORM, SG_EPI_RELU = 0, 1, 2
+SG_EPI_NONE, SG_EPI_NORM, SG_EPI_RELU, SG_EPI_MEAN = 0, 1, 2, 4
+AGGR_AVG, AGGR_MAX, AGGR_MIN, AGGR_SUM = 0, 1, 2, 3
+AGGR = {"mean": AGGR_AVG, "avg": AGGR_AVG, "max": AGGR_MAX, "min": AGGR_MIN, "sum": AGGR_SUM}
+SG_NO_ARG = 0xFFFFFFFF
 LINEAR_NORM_EPILOGUE = 1
 
 
@@ -73,6 +76,9 @@ PROTOTYPES = {
     "roc_sg_forward_planned": (i32, [vp, i32, vp, i64, vp, i64, i32, vp]),
     "roc_sg_forward": (i32, [u32, u32, u64, i32, vp, vp, vp, vp, vp]),
     "roc_sg_backward": (i32, [u32, u32, u64, i32, vp, vp, vp, vp, vp]),
+    "roc_sg_aggr_forward": (i32, [vp, i32, i32, vp, i64, vp, vp, i64, vp, i64, vp]),
+    "roc_sg_arg_backward": (i32, [vp, i32, vp, i64, vp, i64, u32, vp, i64, vp]),
+    "roc_sg_plan_reserve_arg": (i32, [vp, i32]),
     "roc_halo_create": (i32, [u32, u32, u64, vp, vp, C.POINTER(vp)]),
     "roc_halo_destroy": (None, [vp]),
     "roc_halo_size": (u32, [vp]),
@@ -84,6 +90,7 @@ PROTOTYPES = {
     "roc_pack_rows_at": (i32, [i64, i32, vp, vp, vp, i64, vp, i64, vp]),
     "roc_push_rows": (i32, [i64, i32, vp, vp, vp, vp, i64, vp, i32, i64, i32, vp]),
     "roc_indegree_norm": (i32, [u32, u32, u64, i32, vp, vp, i64, vp, i64, vp, vp]),
+    "roc_indegree_div": (i32, [u32, u32, u64, i32, vp, vp, i64, vp, i64, vp]),
     "roc_activation_fwd": (i32, [i64, i32, i32, vp, i64, vp, i64, vp]),
     "roc_activation_bwd": (i32, [i64, i32, i32, vp, i64, vp, i64, vp, i64, i32, vp]),
     "roc_add_fwd": (i32, [i64, i32, vp, i64, vp, i64, vp, i64, vp]),
@@ -123,6 +130,7 @@ PROTOTYPES = {
     "roc_host_linear": (i32, [vp, i32, i32, i32]),
     "roc_host_indegree_norm": (i32, [vp, i32]),
     "roc_host_scatter_gather": (i32, [vp, i32]),
+    "roc_host_scatter_gather_aggr": (i32, [vp, i32, i32]),
     "roc_host_relu": (i32, [vp, i32]),
     "roc_host_sigmoid": (i32, [vp, i32]),
     "roc_host_add": (i32, [vp, i32, i32]),
@@ -155,6 +163,7 @@ PROTOTYPES = {
     "roc_host_metrics": (i32, [vp, vp]),
     "roc_host_profile_sg": (i32, [vp, i32]),
     "roc_host_profile_sg_read": (i32, [vp, i32, vp, vp]),
+    "roc_host_sg_arg": (i32, [vp, i32, vp]),
 }
 
 for _name, (_res, _args) in PROTOTYPES.items():

@@ -76,6 +76,32 @@ k_norm(int64_t rows, int Wq, uint64_t colLeft, const uint64_t* __restrict__ rowE
   }
 }
 
+// out = in / (float)deg with the row-uniform IEEE divide (common.cuh); degree-0 rows give 0
+template <int VEC>
+__global__ void __launch_bounds__(EW_T)
+k_deg_div(int64_t rows, int Wq, uint64_t colLeft, const uint64_t* __restrict__ rowEnd,
+          const float* __restrict__ in, int64_t ldIn, float* __restrict__ out, int64_t ldOut) {
+  const int64_t total = rows * (int64_t)Wq;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total;
+       i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / Wq;
+    const int c = (int)(i - r * Wq);
+    const uint64_t s = (r == 0) ? colLeft : rowEnd[r - 1];
+    const uint32_t deg = (uint32_t)(rowEnd[r] - s);
+    if (VEC == 4) {
+      float v[4] = {0.f, 0.f, 0.f, 0.f};
+      if (deg) {
+        const float4 x = *reinterpret_cast<const float4*>(in + r * ldIn + 4 * c);
+        v[0] = x.x; v[1] = x.y; v[2] = x.z; v[3] = x.w;
+        rowdiv4(v, rowdiv_make((float)deg));
+      }
+      *reinterpret_cast<float4*>(out + r * ldOut + 4 * c) = make_float4(v[0], v[1], v[2], v[3]);
+    } else {
+      out[r * ldOut + c] = deg ? rowdiv(in[r * ldIn + c], rowdiv_make((float)deg)) : 0.f;
+    }
+  }
+}
+
 // ---------------------------------------------------------- generic maps ----
 enum { OP_RELU_F, OP_SIGM_F, OP_RELU_B, OP_SIGM_B, OP_ADD_F, OP_COPY };
 
@@ -624,6 +650,22 @@ extern "C" int roc_indegree_norm(roc_vid_t rowLeft, roc_vid_t rowRight, roc_eid_
     k_norm<4><<<ew_grid(rows * Wq, EW_T), EW_T, 0, st>>>(rows, Wq, colLeft, rowEnd, in, ldIn, out, ldOut, reluOf, ldR);
   } else {
     k_norm<1><<<ew_grid(rows * H, EW_T), EW_T, 0, st>>>(rows, H, colLeft, rowEnd, in, ldIn, out, ldOut, reluOf, ldR);
+  }
+  ROC_LAUNCH_CHECK();
+  return ROC_OK;
+}
+
+extern "C" int roc_indegree_div(roc_vid_t rowLeft, roc_vid_t rowRight, roc_eid_t colLeft, int H,
+                                const roc_eid_t* rowEnd, const float* in, int64_t ldIn, float* out, int64_t ldOut,
+                                roc_stream_t stream) {
+  if (!rowEnd || !in || !out || H <= 0 || rowRight < rowLeft || ldIn < H || ldOut < H) return ROC_ERR_INVALID;
+  const int64_t rows = (int64_t)rowRight - rowLeft + 1;
+  cudaStream_t st = as_stream(stream);
+  if (vec_ok(4, {ldIn, ldOut}, {in, out})) {
+    const int Wq = (H + 3) / 4;
+    k_deg_div<4><<<ew_grid(rows * Wq, EW_T), EW_T, 0, st>>>(rows, Wq, colLeft, rowEnd, in, ldIn, out, ldOut);
+  } else {
+    k_deg_div<1><<<ew_grid(rows * H, EW_T), EW_T, 0, st>>>(rows, H, colLeft, rowEnd, in, ldIn, out, ldOut);
   }
   ROC_LAUNCH_CHECK();
   return ROC_OK;

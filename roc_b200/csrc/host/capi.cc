@@ -87,6 +87,11 @@ int roc_host_linear(roc_host* h, int t, int outDim, int activation) {
 }
 int roc_host_indegree_norm(roc_host* h, int t) { return h->push(h->m().indegree_norm(h->at(t))); }
 int roc_host_scatter_gather(roc_host* h, int t) { return h->push(h->m().scatter_gather(h->at(t))); }
+int roc_host_scatter_gather_aggr(roc_host* h, int t, int aggr) {
+  if (aggr != ROC_AGGR_AVG && aggr != ROC_AGGR_MAX && aggr != ROC_AGGR_MIN && aggr != ROC_AGGR_SUM)
+    ROC_FATAL("roc_host_scatter_gather_aggr: unknown aggregator");
+  return h->push(h->m().scatter_gather(h->at(t), (AggrType)aggr));
+}
 int roc_host_relu(roc_host* h, int t) { return h->push(h->m().relu(h->at(t))); }
 int roc_host_sigmoid(roc_host* h, int t) { return h->push(h->m().sigmoid(h->at(t))); }
 int roc_host_add(roc_host* h, int a, int b) { return h->push(h->m().add(h->at(a), h->at(b))); }
@@ -187,6 +192,20 @@ int roc_host_profile_sg_read(roc_host* h, int maxEntries, int* H, float* ms) {
     H[n] = t.H; ms[n] = e; n++;
   }
   return n;
+}
+int roc_host_sg_arg(roc_host* h, int outTensor, uint32_t* host) {
+  const int region = h->at(outTensor).region;
+  for (GnnOp* op : h->m().layers) {
+    const ScatterGather* sg = dynamic_cast<const ScatterGather*>(op);
+    if (!sg || sg->argRegion < 0 || sg->outputs[0].region != region) continue;
+    RuntimeImpl* rt = h->rt->impl;
+    const TensorImpl& a = rt->t(sg->argRegion);
+    ROC_CHECK(cudaMemcpy2DAsync(host, (size_t)a.H * 4, rt->data(sg->argRegion), (size_t)a.ld * 4, (size_t)a.H * 4,
+                                (size_t)a.rows, cudaMemcpyDeviceToHost, rt->stream));
+    ROC_CHECK(cudaStreamSynchronize(rt->stream));
+    return 0;
+  }
+  return -1;
 }
 int roc_host_metrics(roc_host* h, roc_perf_metrics* out) { *out = h->m().last_metrics(); return 0; }
 

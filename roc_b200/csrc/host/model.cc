@@ -88,8 +88,8 @@ Tensor Model::dropout(const Tensor& _input, float rate, int seed) {
   layers.push_back(op);
   return op->outputs[0];
 }
-Tensor Model::scatter_gather(const Tensor& _input) {
-  GnnOp* op = new ScatterGather(*this, _input);
+Tensor Model::scatter_gather(const Tensor& _input, AggrType aggr) {
+  GnnOp* op = new ScatterGather(*this, _input, aggr);
   layers.push_back(op);
   return op->outputs[0];
 }
@@ -185,15 +185,24 @@ bool Model::init(const Config& config) {
   }
   // scratch: Linear split-K workspace, SG carry slots, the gathered feature matrix
   size_t ws = 0;
-  int maxSg = 0;
+  int maxSg = 0, maxArg = 0;
   for (size_t l = 0; l < layers.size(); l++) {
     if (Linear* lin = as<Linear>(layers[l]))
       ws = std::max(ws, roc_linear_bwd_workspace_bytes(local_rows(), (int)lin->weight.dims[0], (int)lin->weight.dims[1]));
-    if (as<ScatterGather>(layers[l])) maxSg = std::max(maxSg, (int)layers[l]->inputs[0].dims[0]);
+    if (ScatterGather* sg = as<ScatterGather>(layers[l])) {
+      maxSg = std::max(maxSg, (int)sg->inputs[0].dims[0]);
+      if (sg->argRegion >= 0) {
+        maxArg = std::max(maxArg, (int)sg->inputs[0].dims[0]);
+        // the backward reads two tensors at halo rows; the whole-matrix all-gather has one shared buffer
+        if (rt->numParts > 1 && !myGraph.halo)
+          ROC_FATAL("scatter_gather(AGGR_MAX / AGGR_MIN) needs the halo exchange (unset ROC_B200_HALO=0)");
+      }
+    }
   }
   rt->ensure_lin_ws(ws);
   if (maxSg > 0) {
     ROC_CHECK(roc_sg_plan_reserve(myGraph.plan, maxSg));
+    if (maxArg > 0) ROC_CHECK(roc_sg_plan_reserve_arg(myGraph.plan, maxArg));
     if (rt->numParts > 1 && !myGraph.halo) rt->ensure_gather((size_t)myGraph.numNodes * (size_t)round_up4(maxSg));
     if (myGraph.halo) {
       // the tensors a ScatterGather reads get the halo slab appended to their own rows
@@ -207,6 +216,10 @@ bool Model::init(const Config& config) {
         // (gnn.cc:72-74) allows — is re-homed with the halo rows behind its own.
         rt->grow_halo(xin, /*grad=*/false, myGraph.numHalo);
         rt->grow_halo(xout, /*grad=*/true, myGraph.numHalo);
+        // AVG's backward gathers its scaled dOut rows, MAX / MIN's the winner ids: halo rows for them too
+        const ScatterGather* sg = as<ScatterGather>(layers[l]);
+        if (sg->scratch >= 0) rt->grow_halo(rt->t(sg->scratch), /*grad=*/false, myGraph.numHalo);
+        if (sg->argRegion >= 0) rt->grow_halo(rt->t(sg->argRegion), /*grad=*/false, myGraph.numHalo);
       }
       // Exchange by peer writes (roc_push_rows): the slabs exist now and every partition maps the others' copies.
       // ROC_B200_HALO=nccl keeps the staged-rows + NCCL all-to-all-v exchange (cross-check; also the fallback when
@@ -219,13 +232,21 @@ bool Model::init(const Config& config) {
       // ROC_B200_HALO=push | ce forces one.
       rt->p2pCopyEngines = (he && he[0] == 'c') ? true : (he && he[0] == 'p') ? false : rt->numParts == 2;
       for (size_t l = 0; l < layers.size() && rt->p2p; l++) {
-        if (!as<ScatterGather>(layers[l])) continue;
+        const ScatterGather* sg = as<ScatterGather>(layers[l]);
+        if (!sg) continue;
         const int rin = layers[l]->inputs[0].region, rout = layers[l]->outputs[0].region;
         rt->data(rin);
         if (!rt->open_peers(rt->t(rin), false)) { rt->p2p = false; break; }
         if (rt->t(rin).requiresGrad) {
-          rt->grad(rout);
-          if (!rt->open_peers(rt->t(rout), true)) { rt->p2p = false; break; }
+          // the tensor the backward gathers: dOut (SUM, MAX, MIN) or D^-1 dOut (AVG); MAX / MIN also the winner ids
+          const int rg = sg->scratch >= 0 ? sg->scratch : rout;
+          const bool isGrad = sg->scratch < 0;
+          if (isGrad) rt->grad(rg); else rt->data(rg);
+          if (!rt->open_peers(rt->t(rg), isGrad)) { rt->p2p = false; break; }
+          if (sg->argRegion >= 0) {
+            rt->data(sg->argRegion);
+            if (!rt->open_peers(rt->t(sg->argRegion), false)) { rt->p2p = false; break; }
+          }
         }
       }
       if (rt->myPart == 0)
@@ -240,7 +261,7 @@ bool Model::init(const Config& config) {
     Wiring w = wire(layers);
     for (size_t l = 0; l < layers.size(); l++) {
       ScatterGather* sg = as<ScatterGather>(layers[l]);
-      if (!sg) continue;
+      if (!sg || sg->aggr != AGGR_SUM) continue;   // nothing fuses into or across another aggregator
       // upstream: Linear(NONE) -> InDegreeNorm -> SG, each feeding only the next
       int rin = sg->inputs[0].region;
       if (w.producer.count(rin) && w.consumers[rin] == 1) {
@@ -610,14 +631,20 @@ struct PushPipe {
 }  // namespace
 
 // -------------------------------------------------------- ScatterGather -----
-ScatterGather::ScatterGather(const Model& model, const Tensor& _input)
-    : GnnOp(_input), epilogue(0), bwdEpilogue(0), fwdOut(-1), bwdOut(-1) {
+ScatterGather::ScatterGather(const Model& model, const Tensor& _input, AggrType _aggr)
+    : GnnOp(_input), aggr(_aggr), scratch(-1), argRegion(-1), epilogue(0), bwdEpilogue(0), fwdOut(-1), bwdOut(-1) {
   // scattergather.cc:33-37
   ROC_ASSERT(inputs[0].type == Tensor::NODE_TENSOR);
   ROC_ASSERT(inputs[0].numDim == 2);
   ROC_ASSERT(inputs[0].dims[1] == model.myGraph.numNodes);
+  ROC_ASSERT(aggr == AGGR_SUM || aggr == AGGR_AVG || aggr == AGGR_MAX || aggr == AGGR_MIN);
   numOutputs = 1;
-  outputs[0] = model.create_node_tensor<DATATYPE>((int)inputs[0].dims[0]);
+  const int H = (int)inputs[0].dims[0];
+  outputs[0] = model.create_node_tensor<DATATYPE>(H);
+  // per-op buffers, allocated with the op (nothing is allocated inside a step); u32 ids live in a float tensor and
+  // are only ever moved bitwise
+  if (aggr == AGGR_AVG) scratch = model.ctx->new_tensor(model.local_rows(), H, round_up4(H), false, false);
+  if (aggr == AGGR_MAX || aggr == AGGR_MIN) argRegion = model.ctx->new_tensor(model.local_rows(), H, round_up4(H), false, false);
 }
 void ScatterGather::init(const Model&) {}
 
@@ -676,7 +703,17 @@ void ScatterGather::forward(const Model& model) {
   rt->sg_end();
   float* dst = rt->data(outRegion);
   rt->sg_begin(H);
-  ROC_CHECK(roc_sg_forward_planned(model.myGraph.plan, H, src, ldIn, dst, rt->t(outRegion).ld, epilogue, rt->stream));
+  if (aggr == AGGR_MAX || aggr == AGGR_MIN) {
+    // winner ids only when a backward follows
+    const bool wantArg = rt->t(inputs[0].region).requiresGrad && model.mode == MD_MODE_TRAIN;
+    TensorImpl& at = rt->t(argRegion);
+    uint32_t* arg = wantArg ? reinterpret_cast<uint32_t*>(rt->data(argRegion)) : NULL;
+    ROC_CHECK(roc_sg_aggr_forward(model.myGraph.plan, aggr == AGGR_MAX ? ROC_AGGR_MAX : ROC_AGGR_MIN, H, src, ldIn,
+                                  model.myGraph.d_colSrc, dst, rt->t(outRegion).ld, arg, at.ld, rt->stream));
+  } else {
+    const int epi = epilogue | (aggr == AGGR_AVG ? ROC_SG_EPI_MEAN : 0);
+    ROC_CHECK(roc_sg_forward_planned(model.myGraph.plan, H, src, ldIn, dst, rt->t(outRegion).ld, epi, rt->stream));
+  }
   rt->sg_end();
 }
 
@@ -687,6 +724,35 @@ void ScatterGather::backward(const Model& model) {
   const int H = (int)inputs[0].dims[0];
   const int64_t ld = rt->t(outputs[0].region).ld;
   const int dstRegion = bwdOut >= 0 ? bwdOut : inputs[0].region;
+  const Graph& g = model.myGraph;
+  if (aggr == AGGR_AVG) {
+    // dIn = A (D^-1 dOut): scale the dOut rows into the scratch tensor, exchange that, then SUM's gather
+    TensorImpl& sc = rt->t(scratch);
+    ROC_CHECK(roc_indegree_div(g.rowLeft, g.rowRight, g.colLeft, H, g.d_rowEnd, rt->grad(outputs[0].region), ld,
+                               rt->data(scratch), sc.ld, rt->stream));
+    rt->sg_begin(-H);
+    const float* src = gathered(model, rt->data(scratch), sc.ld, H, &sc, false);
+    rt->sg_end();
+    rt->sg_begin(H);
+    ROC_CHECK(roc_sg_forward_planned(g.plan, H, src, sc.ld, rt->grad(dstRegion), rt->t(dstRegion).ld, ROC_SG_EPI_NONE,
+                                     rt->stream));
+    rt->sg_end();
+    return;
+  }
+  if (aggr == AGGR_MAX || aggr == AGGR_MIN) {
+    // dIn[u] = sum over v in in(u) of dOut[v] where arg[v] == u: a gather of dOut and the winner ids at halo rows
+    TensorImpl& at = rt->t(argRegion);
+    rt->sg_begin(-H);
+    const float* src = gathered(model, rt->grad(outputs[0].region), ld, H, &rt->t(outputs[0].region), true);
+    const float* args = gathered(model, rt->data(argRegion), at.ld, H, &at, false);
+    rt->sg_end();
+    ROC_ASSERT(args != src);   // the whole-matrix all-gather's one buffer cannot hold both
+    rt->sg_begin(H);
+    ROC_CHECK(roc_sg_arg_backward(g.plan, H, src, ld, reinterpret_cast<const uint32_t*>(args), at.ld, g.rowLeft,
+                                  rt->grad(dstRegion), rt->t(dstRegion).ld, rt->stream));
+    rt->sg_end();
+    return;
+  }
   // Forward and backward do exactly the same thing, on gradients (scattergather_kernel.cu:168-169)
   rt->sg_begin(-H);
   const float* src = gathered(model, rt->grad(outputs[0].region), ld, H, &rt->t(outputs[0].region), true);

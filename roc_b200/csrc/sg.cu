@@ -57,6 +57,8 @@ struct roc_sg_plan {
   const uint32_t* col = nullptr;  // caller's colSrc
   float* carry = nullptr;         // [numCarries][carryLd]
   size_t carryLd = 0;
+  uint32_t* carryArg = nullptr;   // [numCarries][carryArgLd]  winner ids of the MAX / MIN carry parts
+  size_t carryArgLd = 0;
   uint64_t inRows = 1;            // 1 + largest source id in col: the rows a TMA tensor map of the input spans
   uint32_t* desc = nullptr;       // [numChunks][8] per-chunk start state of the ring kernel (k_chunk_desc)
   int device = 0;
@@ -217,12 +219,15 @@ struct SgParams {
 // The divisor is uniform over the row, so the divide is the row-uniform form of common.cuh
 // (one refined reciprocal, 3 FMAs per element, bit-identical to div.rn): the plain `/` here
 // cost +0.7 ms (H=64) .. +1.8 ms (H=41, zero pad lanes on the slow path) per launch (r1 run 14).
+// MEAN (the AVG aggregator): acc / (float)deg by the same row-uniform IEEE divide; a degree-0 row's sum is
+// +0 and stays so.
 template <int VEC>
 __device__ __forceinline__ void epi_store(typename V<VEC>::T v, typename V<VEC>::T* dst, uint32_t deg, int epi) {
   if (epi & ROC_SG_EPI_NORM) {
     const RowDiv rd = rowdiv_make(sqrtf((float)deg));
     v = V<VEC>::rdiv(v, rd);
   }
+  if ((epi & ROC_SG_EPI_MEAN) && deg) v = V<VEC>::rdiv(v, rowdiv_make((float)deg));
   if (epi & ROC_SG_EPI_RELU) v = V<VEC>::relu(v);
   V<VEC>::st(dst, v);
 }
@@ -851,6 +856,11 @@ template <> struct RV<2> {
       rowdiv4(t, rd, 2);
       v = make_float2(t[0], t[1]);
     }
+    if ((epi & ROC_SG_EPI_MEAN) && deg) {
+      float t[4] = {v.x, v.y, 0.f, 0.f};
+      rowdiv4(t, rowdiv_make((float)deg), 2);
+      v = make_float2(t[0], t[1]);
+    }
     if (epi & ROC_SG_EPI_RELU) v = make_float2(relu_nanprop(v.x), relu_nanprop(v.y));
     *dst = v;
   }
@@ -1161,6 +1171,346 @@ sg_fixup_big_kernel(const SgParams p) {
   }
 }
 
+// ------------------------------------------------ MAX / MIN and their backward ---
+// Kernel A's structure (chunk records, per-row order, rolled segment loop, one store site) with other
+// accumulators:
+//   MAX / MIN  (value, winner id) per element.  The first edge of a segment is taken as is; a later one replaces
+//              the best when it is strictly larger (smaller), or NaN over a non-NaN best — so among equal values
+//              the first edge in CSR order wins and the first NaN wins.  Heavy rows: the owner stores its raw
+//              (value, id), later chunks store theirs into the float carry slots and the u32 carryArg slots, and
+//              sg_aggr_fixup(_big)_kernel merges them in chunk order with the same rule.
+//   ARGBWD     sum of outGrad[src] over the edges whose arg[src] names this row; two rows gathered per edge.
+//              Rows cut at chunk boundaries are plain sums: the SUM fix-up kernels finish them.
+// Algorithmic bytes per launch: MAX / MIN E*(4H+4) + Nloc*(8H+8) (+ the winner ids, E*4, when colGlobal is a
+// separate array); ARGBWD E*(8H+4) + Nloc*(4H+8).
+enum { SG_OP_MAX = 1, SG_OP_MIN = 2, SG_OP_ARGBWD = 3 };
+constexpr uint32_t SG_NO_ARG = 0xFFFFFFFFu;
+
+struct SgAggrParams {
+  SgParams p;              // schedule, in / out / carry; p.ld* and p.Q count VEC-float units
+  const uint32_t* colG;    // MAX / MIN: winner id per edge (parallel to p.col)
+  uint32_t* arg;           // MAX / MIN: [nloc][ldArg] winner ids out (NULL: not stored); ARGBWD: read at col ids
+  uint32_t* carryArg;      // MAX / MIN: [numCarries][ldCA]
+  size_t ldArg, ldCA;      // VEC-u32 units
+  uint32_t rowLeft;        // ARGBWD: global id of local row 0
+};
+
+template <int VEC>
+__device__ __forceinline__ void ldv(float (&a)[VEC], const float* p) {
+  if constexpr (VEC == 4) {
+    const float4 t = *reinterpret_cast<const float4*>(p);
+    a[0] = t.x; a[1] = t.y; a[2] = t.z; a[3] = t.w;
+  } else {
+    a[0] = *p;
+  }
+}
+template <int VEC>
+__device__ __forceinline__ void ldv_nc(float (&a)[VEC], const float* p) {
+  if constexpr (VEC == 4) {
+    const float4 t = __ldg(reinterpret_cast<const float4*>(p));
+    a[0] = t.x; a[1] = t.y; a[2] = t.z; a[3] = t.w;
+  } else {
+    a[0] = __ldg(p);
+  }
+}
+template <int VEC>
+__device__ __forceinline__ void ldu(uint32_t (&a)[VEC], const uint32_t* p) {
+  if constexpr (VEC == 4) {
+    const uint4 t = *reinterpret_cast<const uint4*>(p);
+    a[0] = t.x; a[1] = t.y; a[2] = t.z; a[3] = t.w;
+  } else {
+    a[0] = *p;
+  }
+}
+template <int VEC>
+__device__ __forceinline__ void ldu_nc(uint32_t (&a)[VEC], const uint32_t* p) {
+  if constexpr (VEC == 4) {
+    const uint4 t = __ldg(reinterpret_cast<const uint4*>(p));
+    a[0] = t.x; a[1] = t.y; a[2] = t.z; a[3] = t.w;
+  } else {
+    a[0] = __ldg(p);
+  }
+}
+template <int VEC>
+__device__ __forceinline__ void stv(float* p, const float (&a)[VEC]) {
+  if constexpr (VEC == 4) *reinterpret_cast<float4*>(p) = make_float4(a[0], a[1], a[2], a[3]);
+  else *p = a[0];
+}
+template <int VEC>
+__device__ __forceinline__ void stu(uint32_t* p, const uint32_t (&a)[VEC]) {
+  if constexpr (VEC == 4) *reinterpret_cast<uint4*>(p) = make_uint4(a[0], a[1], a[2], a[3]);
+  else *p = a[0];
+}
+// does candidate c replace the best b (c comes later in CSR order)?
+template <int OP>
+__device__ __forceinline__ bool aggr_better(float c, float b) {
+  return (OP == SG_OP_MAX ? (c > b) : (c < b)) || (c != c && b == b);
+}
+
+template <int OP, int VEC, int L, int NCH, int U, int MINB>
+__global__ void __launch_bounds__(SG_THREADS, MINB)
+sg_aggr_kernel(const SgAggrParams a) {
+  constexpr bool ARG = OP != SG_OP_ARGBWD;
+  constexpr int WPB = SG_THREADS / L;
+  constexpr uint32_t CH = SG_CH;
+  const SgParams& p = a.p;
+  const int lane = threadIdx.x % L;
+  const uint32_t w = blockIdx.x * WPB + threadIdx.x / L;
+  if (w >= p.numChunks) return;
+  const uint32_t* __restrict__ rs = p.rs;
+  const uint32_t* __restrict__ col = p.col;
+
+  bool act[NCH];
+#pragma unroll
+  for (int ch = 0; ch < NCH; ch++) act[ch] = (uint32_t)(lane + ch * L) < p.Q;
+  const uint32_t ce = min(w * CH + CH, p.E);
+  const uint4 dA = __ldg(reinterpret_cast<const uint4*>(p.desc) + 2 * (size_t)w);
+  const uint4 dB = __ldg(reinterpret_cast<const uint4*>(p.desc) + 2 * (size_t)w + 1);
+  if (dB.z & 2u) return;
+  uint32_t cur = dA.z, curS = dA.w, curT = dB.x;
+  const uint32_t e = dA.x, ee = dA.y, r1 = dB.y, carrySlot = dB.w;
+  int kind = (dB.z & 1u) ? 0 : ((curT - curS > CH) ? 2 : 1);
+  uint32_t segEnd = (kind == 1) ? curT : min(curT, ce);
+
+  float acc[NCH][VEC];
+  uint32_t win[NCH][VEC];
+  bool fresh = true;       // no edge of the current segment seen yet (MAX / MIN)
+#pragma unroll
+  for (int ch = 0; ch < NCH; ch++)
+#pragma unroll
+    for (int k = 0; k < VEC; k++) { acc[ch][k] = 0.f; win[ch][k] = SG_NO_ARG; }
+
+  // one store site; a segment with no edge (degree-0 row) stores 0 / SG_NO_ARG
+  auto flush = [&]() {
+    float* dst = (kind == 0) ? static_cast<float*>(p.carry) + (size_t)carrySlot * p.ldC * VEC
+                             : static_cast<float*>(p.out) + (size_t)cur * p.ldOut * VEC;
+    uint32_t* adst = (kind == 0) ? a.carryArg + (size_t)carrySlot * a.ldCA * VEC : a.arg + (size_t)cur * a.ldArg * VEC;
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) {
+      const int c = (lane + ch * L) * VEC;
+      if (act[ch]) {
+        stv<VEC>(dst + c, acc[ch]);
+        if (ARG && a.arg) stu<VEC>(adst + c, win[ch]);
+      }
+#pragma unroll
+      for (int k = 0; k < VEC; k++) { acc[ch][k] = 0.f; win[ch][k] = SG_NO_ARG; }
+    }
+    fresh = true;
+  };
+  auto advance = [&]() {
+    cur += 1; curS = curT; curT = rs[cur + 1];
+    bool heavy = curT - curS > CH;
+    segEnd = heavy ? min(curT, ce) : curT;
+    kind = heavy ? 2 : 1;
+  };
+
+  // lanes past the row's last column read that column (never stored), so no load needs a predicate
+  const float* inl[NCH];
+  const uint32_t* argl[NCH];
+#pragma unroll
+  for (int ch = 0; ch < NCH; ch++) {
+    const uint32_t c = min((uint32_t)(lane + ch * L), p.Q - 1u) * VEC;
+    inl[ch] = static_cast<const float*>(p.in) + c;
+    argl[ch] = ARG ? nullptr : a.arg + c;
+  }
+  const uint64_t ldInF = (uint64_t)p.ldIn * VEC, ldArgU = (uint64_t)a.ldArg * VEC;
+  const uint32_t eLast = ee - 1u;
+#pragma unroll 1
+  for (uint32_t base = e; base < ee; base += U) {
+    const uint32_t cnt = min((uint32_t)U, ee - base);
+    uint32_t srcs[U], gids[U];
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+      const uint32_t ei = min(base + (uint32_t)u, eLast);
+      srcs[u] = __ldg(col + ei);
+      if (ARG) gids[u] = __ldg(a.colG + ei);
+    }
+    float v[U][NCH][VEC];
+    uint32_t av[U][NCH][VEC];
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+#pragma unroll
+      for (int ch = 0; ch < NCH; ch++) {
+        ldv_nc<VEC>(v[u][ch], inl[ch] + srcs[u] * ldInF);
+        if (!ARG) ldu_nc<VEC>(av[u][ch], argl[ch] + srcs[u] * ldArgU);
+      }
+    }
+    uint32_t pos = 0;
+    for (;;) {
+      const uint32_t lim = min(cnt, segEnd - base);
+#pragma unroll
+      for (int u = 0; u < U; u++) {
+        if ((uint32_t)u >= pos && (uint32_t)u < lim) {
+          if constexpr (ARG) {
+#pragma unroll
+            for (int ch = 0; ch < NCH; ch++)
+#pragma unroll
+              for (int k = 0; k < VEC; k++)
+                if (fresh || aggr_better<OP>(v[u][ch][k], acc[ch][k])) { acc[ch][k] = v[u][ch][k]; win[ch][k] = gids[u]; }
+            fresh = false;
+          } else {
+            const uint32_t me = a.rowLeft + cur;
+#pragma unroll
+            for (int ch = 0; ch < NCH; ch++)
+#pragma unroll
+              for (int k = 0; k < VEC; k++)
+                if (av[u][ch][k] == me) acc[ch][k] += v[u][ch][k];   // skipped, not +0: -0 sums stay -0
+          }
+        }
+      }
+      pos = lim;
+      if (pos >= cnt) break;
+      flush();
+      advance();
+    }
+  }
+  flush();
+  while (cur + 1 < r1) { advance(); flush(); }  // trailing zero-degree rows
+}
+
+// One worker per heavy row: merge the owner's partial with the carry parts in chunk order.
+template <int OP, int VEC, int L, int NCH>
+__global__ void __launch_bounds__(SG_THREADS)
+sg_aggr_fixup_kernel(const SgAggrParams a) {
+  constexpr int WPB = SG_THREADS / L;
+  constexpr uint32_t CH = SG_CH;
+  const SgParams& p = a.p;
+  const int lane = threadIdx.x % L;
+  const uint32_t w = blockIdx.x * WPB + threadIdx.x / L;
+  if (w >= p.numHeavy) return;
+  const uint32_t R = p.heavyRows[w];
+  const uint32_t s = p.rs[R], t = p.rs[R + 1];
+  const uint32_t n = (t - 1) / CH - s / CH;
+  const uint32_t slot0 = p.carryIdx[s / CH + 1];
+  float* dst = static_cast<float*>(p.out) + (size_t)R * p.ldOut * VEC;
+  uint32_t* adst = a.arg ? a.arg + (size_t)R * a.ldArg * VEC : nullptr;
+  const float* cv = static_cast<const float*>(p.carry) + (size_t)slot0 * p.ldC * VEC;
+  const uint32_t* ca = a.carryArg + (size_t)slot0 * a.ldCA * VEC;
+#pragma unroll
+  for (int ch = 0; ch < NCH; ch++) {
+    const int c = (lane + ch * L) * VEC;
+    if ((uint32_t)(lane + ch * L) >= p.Q) continue;
+    float best[VEC];
+    uint32_t bw[VEC] = {};
+    ldv<VEC>(best, dst + c);
+    if (adst) ldu<VEC>(bw, adst + c);
+#pragma unroll 4
+    for (uint32_t k = 0; k < n; k++) {
+      float x[VEC];
+      uint32_t xw[VEC] = {};
+      ldv<VEC>(x, cv + (size_t)k * p.ldC * VEC + c);
+      if (adst) ldu<VEC>(xw, ca + (size_t)k * a.ldCA * VEC + c);
+#pragma unroll
+      for (int j = 0; j < VEC; j++)
+        if (aggr_better<OP>(x[j], best[j])) { best[j] = x[j]; bw[j] = xw[j]; }
+    }
+    stv<VEC>(dst + c, best);
+    if (adst) stu<VEC>(adst + c, bw);
+  }
+}
+
+// Rows with more than SG_BIG carries: a CTA per row, the lane groups reduce contiguous blocks of the carries and
+// group 0 merges owner + blocks in order (one column block at a time through shared memory).
+template <int OP, int VEC, int L, int NCH>
+__global__ void __launch_bounds__(SG_THREADS)
+sg_aggr_fixup_big_kernel(const SgAggrParams a) {
+  constexpr int WPB = SG_THREADS / L;
+  constexpr uint32_t CH = SG_CH;
+  __shared__ float sv[WPB][L * VEC];
+  __shared__ uint32_t sw[WPB][L * VEC];
+  const SgParams& p = a.p;
+  const int lane = threadIdx.x % L;
+  const int g = threadIdx.x / L;
+  const uint32_t R = p.bigRows[blockIdx.x];
+  const uint32_t s = p.rs[R], t = p.rs[R + 1];
+  const uint32_t n = (t - 1) / CH - s / CH;
+  const uint32_t slot0 = p.carryIdx[s / CH + 1];
+  const uint32_t per = (n + WPB - 1) / WPB;
+  const uint32_t k0 = min(n, (uint32_t)g * per), k1 = min(n, k0 + per);
+  float* dst = static_cast<float*>(p.out) + (size_t)R * p.ldOut * VEC;
+  uint32_t* adst = a.arg ? a.arg + (size_t)R * a.ldArg * VEC : nullptr;
+  const float* cv = static_cast<const float*>(p.carry) + (size_t)slot0 * p.ldC * VEC;
+  const uint32_t* ca = a.carryArg + (size_t)slot0 * a.ldCA * VEC;
+#pragma unroll 1
+  for (int ch = 0; ch < NCH; ch++) {
+    const int c = (lane + ch * L) * VEC;
+    const bool act = (uint32_t)(lane + ch * L) < p.Q;
+    if (act && k0 < k1) {
+      float best[VEC];
+      uint32_t bw[VEC] = {};
+      ldv<VEC>(best, cv + (size_t)k0 * p.ldC * VEC + c);
+      if (adst) ldu<VEC>(bw, ca + (size_t)k0 * a.ldCA * VEC + c);
+#pragma unroll 1
+      for (uint32_t k = k0 + 1; k < k1; k++) {
+        float x[VEC];
+        uint32_t xw[VEC] = {};
+        ldv<VEC>(x, cv + (size_t)k * p.ldC * VEC + c);
+        if (adst) ldu<VEC>(xw, ca + (size_t)k * a.ldCA * VEC + c);
+#pragma unroll
+        for (int j = 0; j < VEC; j++)
+          if (aggr_better<OP>(x[j], best[j])) { best[j] = x[j]; bw[j] = xw[j]; }
+      }
+#pragma unroll
+      for (int j = 0; j < VEC; j++) { sv[g][lane * VEC + j] = best[j]; sw[g][lane * VEC + j] = bw[j]; }
+    }
+    __syncthreads();
+    if (g == 0 && act) {
+      float best[VEC];
+      uint32_t bw[VEC] = {};
+      ldv<VEC>(best, dst + c);                       // the owner chunk's raw partial
+      if (adst) ldu<VEC>(bw, adst + c);
+      for (int gg = 0; gg < WPB; gg++) {
+        if ((uint32_t)gg * per >= n) break;          // this group and the later ones hold no carries
+#pragma unroll
+        for (int j = 0; j < VEC; j++) {
+          const float x = sv[gg][lane * VEC + j];
+          if (aggr_better<OP>(x, best[j])) { best[j] = x; bw[j] = sw[gg][lane * VEC + j]; }
+        }
+      }
+      stv<VEC>(dst + c, best);
+      if (adst) stu<VEC>(adst + c, bw);
+    }
+    __syncthreads();
+  }
+}
+
+template <int OP, int VEC, int L, int NCH, int U, int MINB>
+static int launch_aggr_cfg(const SgAggrParams& a, cudaStream_t st) {
+  constexpr int WPB = SG_THREADS / L;
+  constexpr int UU = (OP == SG_OP_ARGBWD && U > 1) ? U / 2 : U;   // two rows per edge: half the edges in flight
+  // cut rows of ARGBWD are plain sums: SUM's fix-up kernels (the same instantiations SUM launches) finish them
+  const SgParams& p = a.p;
+  if (p.numChunks) {
+    sg_aggr_kernel<OP, VEC, L, NCH, UU, MINB><<<(p.numChunks + WPB - 1) / WPB, SG_THREADS, 0, st>>>(a);
+    ROC_LAUNCH_CHECK();
+  }
+  if (p.numHeavy) {
+    const unsigned grid = (p.numHeavy + WPB - 1) / WPB;
+    if constexpr (OP == SG_OP_ARGBWD) sg_fixup_kernel<VEC, L, NCH, U><<<grid, SG_THREADS, 0, st>>>(p);
+    else sg_aggr_fixup_kernel<OP, VEC, L, NCH><<<grid, SG_THREADS, 0, st>>>(a);
+    ROC_LAUNCH_CHECK();
+  }
+  if (p.numBig) {
+    if constexpr (OP == SG_OP_ARGBWD) sg_fixup_big_kernel<VEC, L, NCH, U><<<p.numBig, SG_THREADS, 0, st>>>(p);
+    else sg_aggr_fixup_big_kernel<OP, VEC, L, NCH><<<p.numBig, SG_THREADS, 0, st>>>(a);
+    ROC_LAUNCH_CHECK();
+  }
+  return ROC_OK;
+}
+
+template <int OP, int VEC>
+static int dispatch_aggr(const SgAggrParams& a, cudaStream_t st) {
+  const uint32_t Q = a.p.Q;
+  if (Q <= 4) return launch_aggr_cfg<OP, VEC, 4, 1, 4, 4>(a, st);
+  if (Q <= 8) return launch_aggr_cfg<OP, VEC, 8, 1, 8, 3>(a, st);
+  if (Q <= 16) return launch_aggr_cfg<OP, VEC, 16, 1, 8, 3>(a, st);
+  if (Q <= 32) return launch_aggr_cfg<OP, VEC, 32, 1, 8, 3>(a, st);
+  if (Q <= 64) return launch_aggr_cfg<OP, VEC, 32, 2, 4, 2>(a, st);
+  if (Q <= 128) return launch_aggr_cfg<OP, VEC, 32, 4, 2, 2>(a, st);
+  if (Q <= 256) return launch_aggr_cfg<OP, VEC, 32, 8, 1, 1>(a, st);
+  return ROC_ERR_UNSUPPORTED;
+}
+
 // Variant A keeps the gathers in registers, variant C stages them in shared memory with
 // cp.async; C wins once a row needs two or more float4 per lane at L = 32 (H > 128).
 // ROC_SG_VARIANT=a|c forces one (experiments / cross-checks).
@@ -1384,18 +1734,26 @@ static int pick_variant(uint32_t Q, bool vec) {
 // init-time call).  A launch that still finds them too small grows them on its own stream with stream-ordered
 // allocation: the old buffer is returned in stream order, after the launches that used it — no device
 // synchronisation in the middle of a step.
-static int ensure_carry(roc_sg_plan* plan, size_t ldFloats, cudaStream_t st, bool inStream) {
-  if (plan->numCarries == 0 || ldFloats <= plan->carryLd) return ROC_OK;
-  if (plan->carry) {
-    if (inStream) ROC_CUDA(cudaFreeAsync(plan->carry, st));
-    else { ROC_CUDA(cudaDeviceSynchronize()); ROC_CUDA(cudaFree(plan->carry)); }
-    plan->carry = nullptr; plan->carryLd = 0;
+template <typename W>
+static int grow_carry(const roc_sg_plan* plan, W*& buf, size_t& have, size_t ld, cudaStream_t st, bool inStream) {
+  if (plan->numCarries == 0 || ld <= have) return ROC_OK;
+  if (buf) {
+    if (inStream) ROC_CUDA(cudaFreeAsync(buf, st));
+    else { ROC_CUDA(cudaDeviceSynchronize()); ROC_CUDA(cudaFree(buf)); }
+    buf = nullptr; have = 0;
   }
-  const size_t bytes = (size_t)plan->numCarries * ldFloats * sizeof(float);
-  cudaError_t e = inStream ? cudaMallocAsync((void**)&plan->carry, bytes, st) : cudaMalloc((void**)&plan->carry, bytes);
-  if (e != cudaSuccess) { plan->carry = nullptr; plan->carryLd = 0; return (int)e; }
-  plan->carryLd = ldFloats;
+  const size_t bytes = (size_t)plan->numCarries * ld * sizeof(W);
+  cudaError_t e = inStream ? cudaMallocAsync((void**)&buf, bytes, st) : cudaMalloc((void**)&buf, bytes);
+  if (e != cudaSuccess) { buf = nullptr; have = 0; return (int)e; }
+  have = ld;
   return ROC_OK;
+}
+static int ensure_carry(roc_sg_plan* plan, size_t ldFloats, cudaStream_t st, bool inStream) {
+  return grow_carry(plan, plan->carry, plan->carryLd, ldFloats, st, inStream);
+}
+// the u32 twins of the carry slots: winner ids of the MAX / MIN carry parts
+static int ensure_carry_arg(roc_sg_plan* plan, size_t ld, cudaStream_t st, bool inStream) {
+  return grow_carry(plan, plan->carryArg, plan->carryArgLd, ld, st, inStream);
 }
 
 }  // namespace roc
@@ -1490,6 +1848,7 @@ done:
 extern "C" void roc_sg_plan_destroy(roc_sg_plan* pl) {
   if (!pl) return;
   cudaFree(pl->rs); cudaFree(pl->firstRow); cudaFree(pl->carryIdx); cudaFree(pl->heavyRows); cudaFree(pl->bigRows); cudaFree(pl->carry); cudaFree(pl->desc);
+  cudaFree(pl->carryArg);
   delete pl;
 }
 
@@ -1511,6 +1870,7 @@ extern "C" int roc_sg_forward_planned(const roc_sg_plan* plc, int H, const float
                                       float* out, int64_t ldOut, int epilogue, roc_stream_t stream) {
   roc_sg_plan* pl = const_cast<roc_sg_plan*>(plc);
   if (!pl || H <= 0 || !in || !out || ldIn < H || ldOut < H) return ROC_ERR_INVALID;
+  if ((epilogue & ROC_SG_EPI_MEAN) && (epilogue & ROC_SG_EPI_NORM)) return ROC_ERR_INVALID;
   cudaStream_t st = as_stream(stream);
   const bool vec = (ldIn % 4 == 0) && (ldOut % 4 == 0) && aligned16(in) && aligned16(out);
   // column blocks: the widest kernel covers 256 T-columns (1024 floats vectorised, 256 scalar);
@@ -1563,6 +1923,74 @@ extern "C" int roc_sg_forward_planned(const roc_sg_plan* plc, int H, const float
     if (rc != ROC_OK) return rc;
   }
   return ROC_OK;
+}
+
+// MAX / MIN forward and their backward: the register kernel in column blocks of up to 1024 floats (256 on the
+// scalar path)
+static int aggr_run(roc_sg_plan* pl, int op, int H, const float* in, int64_t ldIn, const uint32_t* colG, float* out,
+                    int64_t ldOut, uint32_t* arg, int64_t ldArg, uint32_t rowLeft, cudaStream_t st) {
+  const bool vec = (ldIn % 4 == 0) && (ldOut % 4 == 0) && aligned16(in) && aligned16(out) &&
+                   (!arg || ((ldArg % 4 == 0) && aligned16(arg)));
+  const int blockCols = vec ? 1024 : 256;
+  const size_t need = ((size_t)(H < blockCols ? H : blockCols) + 3) / 4 * 4;
+  int rc = ensure_carry(pl, need, st, true);
+  if (rc != ROC_OK) return rc;
+  if (op != SG_OP_ARGBWD && arg) {
+    rc = ensure_carry_arg(pl, need, st, true);
+    if (rc != ROC_OK) return rc;
+  }
+  for (int c0 = 0; c0 < H; c0 += blockCols) {
+    const int hb = (H - c0 < blockCols) ? H - c0 : blockCols;
+    SgAggrParams a;
+    SgParams& p = a.p;
+    p.rs = pl->rs; p.firstRow = pl->firstRow; p.carryIdx = pl->carryIdx; p.heavyRows = pl->heavyRows; p.bigRows = pl->bigRows;
+    p.col = pl->col; p.in = in + c0; p.out = out + c0; p.carry = pl->carry;
+    p.E = pl->E; p.numChunks = pl->numChunks; p.numHeavy = pl->numHeavy; p.numBig = pl->numBig; p.epi = 0;
+    p.dense = 0; p.desc = pl->desc; p.nloc = pl->nloc;
+    a.colG = colG ? colG : pl->col;
+    a.arg = arg ? arg + c0 : nullptr;
+    a.carryArg = pl->carryArg;
+    a.rowLeft = rowLeft;
+    const size_t vw = vec ? 4 : 1;
+    p.ldIn = (size_t)ldIn / vw; p.ldOut = (size_t)ldOut / vw; p.ldC = pl->carryLd / vw;
+    a.ldArg = (size_t)ldArg / vw; a.ldCA = pl->carryArgLd / vw;
+    p.Q = vec ? ((uint32_t)hb + 3) / 4 : (uint32_t)hb;
+    if (vec) {
+      rc = op == SG_OP_MAX ? dispatch_aggr<SG_OP_MAX, 4>(a, st)
+         : op == SG_OP_MIN ? dispatch_aggr<SG_OP_MIN, 4>(a, st) : dispatch_aggr<SG_OP_ARGBWD, 4>(a, st);
+    } else {
+      rc = op == SG_OP_MAX ? dispatch_aggr<SG_OP_MAX, 1>(a, st)
+         : op == SG_OP_MIN ? dispatch_aggr<SG_OP_MIN, 1>(a, st) : dispatch_aggr<SG_OP_ARGBWD, 1>(a, st);
+    }
+    if (rc != ROC_OK) return rc;
+  }
+  return ROC_OK;
+}
+
+extern "C" int roc_sg_aggr_forward(const roc_sg_plan* plc, int aggr, int H, const float* in, int64_t ldIn,
+                                   const roc_vid_t* colGlobal, float* out, int64_t ldOut, uint32_t* arg,
+                                   int64_t ldArg, roc_stream_t stream) {
+  roc_sg_plan* pl = const_cast<roc_sg_plan*>(plc);
+  if (!pl || H <= 0 || !in || !out || ldIn < H || ldOut < H || (arg && ldArg < H)) return ROC_ERR_INVALID;
+  if (aggr != ROC_AGGR_MAX && aggr != ROC_AGGR_MIN) return ROC_ERR_INVALID;
+  return aggr_run(pl, aggr == ROC_AGGR_MAX ? SG_OP_MAX : SG_OP_MIN, H, in, ldIn, colGlobal, out, ldOut, arg, ldArg, 0u,
+                  as_stream(stream));
+}
+
+extern "C" int roc_sg_arg_backward(const roc_sg_plan* plc, int H, const float* outGrad, int64_t ldG,
+                                   const uint32_t* arg, int64_t ldArg, roc_vid_t rowLeft, float* inGrad,
+                                   int64_t ldIn, roc_stream_t stream) {
+  roc_sg_plan* pl = const_cast<roc_sg_plan*>(plc);
+  if (!pl || H <= 0 || !outGrad || !arg || !inGrad || ldG < H || ldArg < H || ldIn < H) return ROC_ERR_INVALID;
+  return aggr_run(pl, SG_OP_ARGBWD, H, outGrad, ldG, nullptr, inGrad, ldIn, const_cast<uint32_t*>(arg), ldArg, rowLeft,
+                  as_stream(stream));
+}
+
+extern "C" int roc_sg_plan_reserve_arg(roc_sg_plan* pl, int maxH) {
+  if (!pl || maxH <= 0) return ROC_ERR_INVALID;
+  const size_t ld = ((size_t)maxH + 3) / 4 * 4;
+  const int rc = ensure_carry(pl, ld, nullptr, false);
+  return rc != ROC_OK ? rc : ensure_carry_arg(pl, ld, nullptr, false);
 }
 
 extern "C" int roc_sg_forward(roc_vid_t rowLeft, roc_vid_t rowRight, roc_eid_t colLeft, int H,

@@ -66,6 +66,36 @@ class SgPlan:
                                          _stream()), "roc_sg_forward_planned")
         return out
 
+    def reserve_arg(self, max_h):
+        check(lib.roc_sg_plan_reserve_arg(self.handle, int(max_h)), "roc_sg_plan_reserve_arg")
+
+    def aggr_forward(self, x, aggr, col_global=None, out=None, arg=None, want_arg=True):
+        """MAX / MIN (aggr = "max" | "min" or _lib.AGGR_*): returns (out, arg); arg is a [nloc][H] int32 view of
+        the u32 winner ids (global vertex ids; -1 = 0xFFFFFFFF for degree-0 rows), or None with want_arg=False."""
+        aggr = _lib.AGGR[aggr] if isinstance(aggr, str) else int(aggr)
+        nloc = self.row_right - self.row_left + 1
+        h = x.shape[1]
+        vec = _ld(x) % 4 == 0
+        if out is None:
+            out = padded(nloc, h, x.device) if vec else torch.empty((nloc, h), device=x.device)
+        if arg is None and want_arg:
+            arg = padded(nloc, h, x.device, dtype=torch.int32) if vec else torch.empty((nloc, h), device=x.device,
+                                                                                     dtype=torch.int32)
+        check(lib.roc_sg_aggr_forward(self.handle, aggr, h, _ptr(x), _ld(x), _ptr(col_global), _ptr(out), _ld(out),
+                                      _ptr(arg), _ld(arg) if arg is not None else 0, _stream()),
+              "roc_sg_aggr_forward")
+        return out, arg
+
+    def arg_backward(self, gy, arg, out=None):
+        """dIn[u] = sum over the plan's edges (u <- v) of gy[v] where arg[v] == row_left + u."""
+        nloc = self.row_right - self.row_left + 1
+        h = gy.shape[1]
+        if out is None:
+            out = padded(nloc, h, gy.device) if _ld(gy) % 4 == 0 else torch.empty((nloc, h), device=gy.device)
+        check(lib.roc_sg_arg_backward(self.handle, h, _ptr(gy), _ld(gy), _ptr(arg), _ld(arg), self.row_left,
+                                      _ptr(out), _ld(out), _stream()), "roc_sg_arg_backward")
+        return out
+
     def close(self):
         if self.handle:
             lib.roc_sg_plan_destroy(self.handle)
@@ -111,6 +141,15 @@ def indegree_norm(row_left, row_right, col_left, row_end, x, out=None, relu_mask
         out = torch.empty_like(x) if x.is_contiguous() else padded(x.shape[0], x.shape[1], x.device)
     check(lib.roc_indegree_norm(row_left, row_right, col_left, x.shape[1], _ptr(row_end), _ptr(x), _ld(x), _ptr(out),
                                 _ld(out), _ptr(relu_mask_of), _stream()), "roc_indegree_norm")
+    return out
+
+
+def indegree_div(row_left, row_right, col_left, row_end, x, out=None):
+    """out = x / (float)deg per row (IEEE division; degree-0 rows give 0)."""
+    if out is None:
+        out = torch.empty_like(x) if x.is_contiguous() else padded(x.shape[0], x.shape[1], x.device)
+    check(lib.roc_indegree_div(row_left, row_right, col_left, x.shape[1], _ptr(row_end), _ptr(x), _ld(x), _ptr(out),
+                               _ld(out), _stream()), "roc_indegree_div")
     return out
 
 

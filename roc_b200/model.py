@@ -92,8 +92,18 @@ class Model:
     def indegree_norm(self, t):
         return lib.roc_host_indegree_norm(self.h, t)
 
-    def scatter_gather(self, t):
-        return lib.roc_host_scatter_gather(self.h, t)
+    def scatter_gather(self, t, aggr="sum"):
+        """aggr: "sum" (the reference's ScatterGather), "mean", "max" or "min"."""
+        if aggr == "sum":
+            return lib.roc_host_scatter_gather(self.h, t)
+        return lib.roc_host_scatter_gather_aggr(self.h, t, _lib.AGGR[aggr])
+
+    def sg_arg(self, t):
+        """Winner ids (u32, global vertex ids) of the max / min scatter_gather whose output is `t`, own rows."""
+        rows, hidden, _ = self.tensor_shape(t)
+        out = np.empty((rows, hidden), dtype=np.uint32)
+        check(lib.roc_host_sg_arg(self.h, t, out.ctypes.data), "roc_host_sg_arg")
+        return out
 
     def relu(self, t):
         return lib.roc_host_relu(self.h, t)
@@ -279,3 +289,34 @@ def build_sage_mean(model, layers, dropout_rate, lr=0.01, weight_decay=0.05):
     model.adam(lr, weight_decay)
     model.init()
     return {"input": x, "label": label, "mask": mask, "logits": t, "relu_outs": relu_outs}
+
+
+def build_sage(model, layers, dropout_rate, aggr="mean", lr=0.01, weight_decay=0.05):
+    """GraphSAGE with a native aggregator ("mean", "max", "min" or "sum"): build_sage_mean's wiring
+
+        D  = dropout(t)
+        t  = add(scatter_gather(linear(D, d_i), aggr), linear(D, d_i))     # neighbours + the root / self weight
+        t  = relu(t)                                                          # all but the last layer
+
+    with the aggregation done by one ScatterGather (mean: one IEEE division of the sum by the in-degree).
+    "sage_outs" are the aggregation outputs (for max / min: where Model.sg_arg reads the winner ids)."""
+    L = len(layers)
+    x = model.create_node_tensor(layers[0])
+    label = model.create_node_tensor(layers[-1])
+    mask = model.create_node_tensor(1, is_int=True)
+    t = x
+    relu_outs, sage_outs = [], []
+    for i in range(1, L):
+        d = model.dropout(t, dropout_rate)
+        nb = model.linear(d, layers[i], _lib.AC_MODE_NONE)
+        nb = model.scatter_gather(nb, aggr)
+        sage_outs.append(nb)
+        root = model.linear(d, layers[i], _lib.AC_MODE_NONE)
+        t = model.add(nb, root)
+        if i != L - 1:
+            t = model.relu(t)
+            relu_outs.append(t)
+    model.softmax_cross_entropy(t, label, mask)
+    model.adam(lr, weight_decay)
+    model.init()
+    return {"input": x, "label": label, "mask": mask, "logits": t, "relu_outs": relu_outs, "sage_outs": sage_outs}
