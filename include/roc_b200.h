@@ -185,6 +185,49 @@ int roc_sg_arg_backward(const roc_sg_plan* plan, int H, const float* outGrad, in
  * roc_sg_plan_reserve for the float ones, which it also reserves), for widths up to maxH. */
 int roc_sg_plan_reserve_arg(roc_sg_plan* plan, int maxH);
 
+/* Graph attention (GAT, one layer, K heads) over the plan's rows.  h is [rows][H] with H = K*F, head k the columns
+ * [kF, (k+1)F); attW is the op's parameter [2][H]: row 0 a_src, row 1 a_dst.  Per-node tensors (K <= 8):
+ *   att [rows][ldAtt >= 2K]: s_src[r][k] = <h[r, k-block], a_src[k-block]> at column k, s_dst at column K + k
+ *   bst [rows][ldB >= 2K]:   lse[r][k] at column k (the forward), c[r][k] = <dOut[r, k-block], out[r, k-block]> at
+ *                            column K + k (the backward)
+ * For a row v, its in-edges u (CSR order) and head k:
+ *   e = LeakyReLU(s_src[u][k] + s_dst[v][k], slope);  lse[v][k] = max e + log sum exp(e - max e)
+ *   alpha = expf(e - lse[v][k]);  out[v, k-block] = sum_u alpha h[u, k-block]
+ * A degree-0 row has out = 0 and lse = 0.  alpha is recomputed wherever it is needed, by one device function.
+ * Tensors the gathers index (h, att, bst, outGrad) are indexed by the plan's col ids, and their rows 0 .. nloc-1
+ * are the plan's own rows ([own | halo] in the multi-GPU engine; the whole matrix with rowLeft = 0 otherwise).
+ * Supported: K in {1, 2, 4, 8}, 1 <= H <= 256, and F % 4 == 0 when K > 1; anything else is ROC_ERR_UNSUPPORTED.
+ * Pad columns (past H) enter no dot and no sum.  No atomics: every result is bit-reproducible. */
+int roc_gat_supported(int H, int heads);
+/* Size the plan's carry slots for the widest GAT pass at width H (init time; nothing is allocated in a step). */
+int roc_gat_plan_reserve(roc_sg_plan* plan, int H, int heads);
+/* att[r] = (s_src[r] | s_dst[r]) for rows 0 .. rows-1. */
+int roc_gat_scores(int64_t rows, int H, int heads, const float* h, int64_t ldH, const float* attW, float* att,
+                   int64_t ldAtt, roc_stream_t stream);
+/* lse (into bst's first K columns of the own rows) in one pass over the edges, then out in a second. */
+int roc_gat_forward(const roc_sg_plan* plan, int H, int heads, float slope, const float* h, int64_t ldH,
+                    const float* att, int64_t ldAtt, float* bst, int64_t ldB, float* out, int64_t ldOut,
+                    roc_stream_t stream);
+/* c[r][k] = <outGrad[r, k-block], out[r, k-block]> into bst's columns K .. 2K-1, rows 0 .. rows-1. */
+int roc_gat_bwd_c(int64_t rows, int H, int heads, const float* outGrad, int64_t ldG, const float* out,
+                  int64_t ldOut, float* bst, int64_t ldB, roc_stream_t stream);
+/* The backward gather.  Row u walks its in-edges v (which, with a symmetric in-edge CSR, are the rows u feeds;
+ * quirk Q1 as for every aggregator's backward):
+ *   inGrad[u]     = sum_v alpha[v<-u] outGrad[v]                                                (overwritten)
+ *   ds[u][k]      = sum_v alpha[v<-u,k] (<outGrad[v], h[u]>_k - c[v][k]) LeakyReLU'(s_src[u][k] + s_dst[v][k])
+ *   ds[u][K + k]  = sum_v alpha[u<-v,k] (<outGrad[u], h[v]>_k - c[u][k]) LeakyReLU'(s_src[v][k] + s_dst[u][k])
+ * with LeakyReLU'(z) = 1 if z > 0 else slope.  ds is [nloc][ldDs >= 2K]. */
+int roc_gat_backward(const roc_sg_plan* plan, int H, int heads, float slope, const float* h, int64_t ldH,
+                     const float* att, int64_t ldAtt, const float* bst, int64_t ldB, const float* outGrad,
+                     int64_t ldG, float* inGrad, int64_t ldIn, float* ds, int64_t ldDs, roc_stream_t stream);
+/* inGrad[r][j] += ds[r][k(j)] a_src[j] + ds[r][K + k(j)] a_dst[j]  (rows 0 .. rows-1), and
+ * attGrad[0][j] = sum_r ds[r][k(j)] h[r][j], attGrad[1][j] = sum_r ds[r][K + k(j)] h[r][j] (overwritten), as
+ * fixed row blocks summed in block order.  workspace: roc_gat_finish_workspace_bytes(H). */
+size_t roc_gat_finish_workspace_bytes(int H);
+int roc_gat_bwd_finish(int64_t rows, int H, int heads, const float* h, int64_t ldH, const float* attW,
+                       const float* ds, int64_t ldDs, float* inGrad, int64_t ldIn, float* attGrad, void* workspace,
+                       size_t workspaceBytes, roc_stream_t stream);
+
 /* ----------------------------------------------------------------- halo --- */
 
 /* Boundary-node structures of one partition (multi-GPU).  The reference hands every

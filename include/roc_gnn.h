@@ -187,6 +187,13 @@ public:
    * a symmetric in-edge CSR without duplicate edges, like SUM's (quirk Q1).  Only SUM ops take part in the
    * epilogue fusions. */
   Tensor scatter_gather(const Tensor& _input, AggrType aggr = AGGR_SUM);
+  /* Graph attention (GAT, Velickovic et al. 2018) with `heads` heads over the node tensor _input of width
+   * H = heads * F: out[v, k-block] = sum over in-edges u of alpha[v<-u,k] _input[u, k-block], alpha the softmax over
+   * v's in-edges of LeakyReLU(<h[u], a_src[k]> + <h[v], a_dst[k]>, negativeSlope) per head, heads concatenated.
+   * Owns one parameter [2][H] (row 0 a_src, row 1 a_dst), Glorot-initialised and trained like a Linear weight.
+   * Supported: heads in {1, 2, 4, 8}, H <= 256 and F % 4 == 0 when heads > 1.  The backward assumes a symmetric
+   * in-edge CSR (quirk Q1).  Takes part in no epilogue fusion. */
+  Tensor graph_attention(const Tensor& _input, int heads, float negativeSlope = 0.2f);
   void softmax_cross_entropy(const Tensor& logits, const Tensor& labels, const Tensor& mask);
   Tensor indegree_norm(const Tensor& _input);
   Tensor linear(const Tensor& _input, int outDim, ActiMode activation, Initializer* initializer = NULL);
@@ -259,6 +266,21 @@ public:
   int epilogue;      /* ROC_SG_EPI_* the forward store applies (set by Model::init fusion) */
   int bwdEpilogue;   /* same for the backward launch */
   int fwdOut, bwdOut;/* region the fused forward / backward writes (-1: own output / input grad) */
+};
+
+class GraphAttention : public GnnOp {  /* not in the reference */
+public:
+  GraphAttention(const Model& model, const Tensor& input, int heads, float slope);
+  virtual void init(const Model& model);
+  virtual void forward(const Model& model);
+  virtual void backward(const Model& model);
+  int heads;
+  float slope;
+  Tensor weight;      /* [2][H]: a_src, a_dst */
+  int attRegion;      /* per-node s_src | s_dst [rows (+ halo)][round_up4(2 heads)] */
+  int bstRegion;      /* per-node lse | c, same shape */
+  int dsRegion;       /* backward: ds_src | ds_dst of the own rows */
+  void* work;         /* backward: the da partials (roc_gat_finish_workspace_bytes) */
 };
 
 class InDegreeNorm : public GnnOp {  /* gnn.h:244-261, graphnorm.cc */

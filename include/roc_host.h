@@ -42,6 +42,8 @@ int roc_host_indegree_norm(roc_host* h, int t);
 int roc_host_scatter_gather(roc_host* h, int t);
 /* Model::scatter_gather(t, aggr) with aggr = ROC_AGGR_AVG | _MAX | _MIN | _SUM (roc_b200.h). */
 int roc_host_scatter_gather_aggr(roc_host* h, int t, int aggr);
+/* Model::graph_attention(t, heads, slope): GAT with `heads` heads over tensor t (roc_b200.h's roc_gat_*). */
+int roc_host_graph_attention(roc_host* h, int t, int heads, float slope);
 int roc_host_relu(roc_host* h, int t);
 int roc_host_sigmoid(roc_host* h, int t);
 int roc_host_add(roc_host* h, int a, int b);
@@ -86,6 +88,10 @@ int roc_host_profile_sg_read(roc_host* h, int maxEntries, int* H, float* ms);
  * MAX / MIN scatter_gather whose output is tensor `outTensor`, for this partition's own rows, as the latest
  * training-mode forward left them.  -1 if that tensor is not the output of such an op. */
 int roc_host_sg_arg(roc_host* h, int outTensor, uint32_t* host);
+/* Test hooks of the graph_attention whose output is tensor `outTensor` (-1 if there is none): its lse
+ * ([rows][heads], own rows, as the latest forward left them), and the parameter index of its [2][H] att weight. */
+int roc_host_gat_lse(roc_host* h, int outTensor, float* host);
+int roc_host_gat_param(roc_host* h, int outTensor);
 
 #ifdef __cplusplus
 }

@@ -79,6 +79,14 @@ PROTOTYPES = {
     "roc_sg_aggr_forward": (i32, [vp, i32, i32, vp, i64, vp, vp, i64, vp, i64, vp]),
     "roc_sg_arg_backward": (i32, [vp, i32, vp, i64, vp, i64, u32, vp, i64, vp]),
     "roc_sg_plan_reserve_arg": (i32, [vp, i32]),
+    "roc_gat_supported": (i32, [i32, i32]),
+    "roc_gat_plan_reserve": (i32, [vp, i32, i32]),
+    "roc_gat_scores": (i32, [i64, i32, i32, vp, i64, vp, vp, i64, vp]),
+    "roc_gat_forward": (i32, [vp, i32, i32, f32, vp, i64, vp, i64, vp, i64, vp, i64, vp]),
+    "roc_gat_bwd_c": (i32, [i64, i32, i32, vp, i64, vp, i64, vp, i64, vp]),
+    "roc_gat_backward": (i32, [vp, i32, i32, f32, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp]),
+    "roc_gat_finish_workspace_bytes": (sz, [i32]),
+    "roc_gat_bwd_finish": (i32, [i64, i32, i32, vp, i64, vp, vp, i64, vp, i64, vp, vp, sz, vp]),
     "roc_halo_create": (i32, [u32, u32, u64, vp, vp, C.POINTER(vp)]),
     "roc_halo_destroy": (None, [vp]),
     "roc_halo_size": (u32, [vp]),
@@ -131,6 +139,7 @@ PROTOTYPES = {
     "roc_host_indegree_norm": (i32, [vp, i32]),
     "roc_host_scatter_gather": (i32, [vp, i32]),
     "roc_host_scatter_gather_aggr": (i32, [vp, i32, i32]),
+    "roc_host_graph_attention": (i32, [vp, i32, i32, f32]),
     "roc_host_relu": (i32, [vp, i32]),
     "roc_host_sigmoid": (i32, [vp, i32]),
     "roc_host_add": (i32, [vp, i32, i32]),
@@ -164,6 +173,8 @@ PROTOTYPES = {
     "roc_host_profile_sg": (i32, [vp, i32]),
     "roc_host_profile_sg_read": (i32, [vp, i32, vp, vp]),
     "roc_host_sg_arg": (i32, [vp, i32, vp]),
+    "roc_host_gat_lse": (i32, [vp, i32, vp]),
+    "roc_host_gat_param": (i32, [vp, i32]),
 }
 
 for _name, (_res, _args) in PROTOTYPES.items():

@@ -92,6 +92,9 @@ int roc_host_scatter_gather_aggr(roc_host* h, int t, int aggr) {
     ROC_FATAL("roc_host_scatter_gather_aggr: unknown aggregator");
   return h->push(h->m().scatter_gather(h->at(t), (AggrType)aggr));
 }
+int roc_host_graph_attention(roc_host* h, int t, int heads, float slope) {
+  return h->push(h->m().graph_attention(h->at(t), heads, slope));
+}
 int roc_host_relu(roc_host* h, int t) { return h->push(h->m().relu(h->at(t))); }
 int roc_host_sigmoid(roc_host* h, int t) { return h->push(h->m().sigmoid(h->at(t))); }
 int roc_host_add(roc_host* h, int a, int b) { return h->push(h->m().add(h->at(a), h->at(b))); }
@@ -205,6 +208,32 @@ int roc_host_sg_arg(roc_host* h, int outTensor, uint32_t* host) {
     ROC_CHECK(cudaStreamSynchronize(rt->stream));
     return 0;
   }
+  return -1;
+}
+static const GraphAttention* gat_of(roc_host* h, int outTensor) {
+  const int region = h->at(outTensor).region;
+  for (GnnOp* op : h->m().layers) {
+    const GraphAttention* ga = dynamic_cast<const GraphAttention*>(op);
+    if (ga && ga->outputs[0].region == region) return ga;
+  }
+  return nullptr;
+}
+int roc_host_gat_lse(roc_host* h, int outTensor, float* host) {
+  const GraphAttention* ga = gat_of(h, outTensor);
+  if (!ga) return -1;
+  RuntimeImpl* rt = h->rt->impl;
+  const TensorImpl& b = rt->t(ga->bstRegion);
+  ROC_CHECK(cudaMemcpy2DAsync(host, (size_t)ga->heads * 4, rt->data(ga->bstRegion), (size_t)b.ld * 4,
+                              (size_t)ga->heads * 4, (size_t)b.rows, cudaMemcpyDeviceToHost, rt->stream));
+  ROC_CHECK(cudaStreamSynchronize(rt->stream));
+  return 0;
+}
+int roc_host_gat_param(roc_host* h, int outTensor) {
+  const GraphAttention* ga = gat_of(h, outTensor);
+  if (!ga) return -1;
+  const std::vector<Tensor>& ps = h->m().parameters;
+  for (size_t p = 0; p < ps.size(); p++)
+    if (ps[p].region == ga->weight.region) return (int)p;
   return -1;
 }
 int roc_host_metrics(roc_host* h, roc_perf_metrics* out) { *out = h->m().last_metrics(); return 0; }

@@ -93,6 +93,12 @@ Tensor Model::scatter_gather(const Tensor& _input, AggrType aggr) {
   layers.push_back(op);
   return op->outputs[0];
 }
+Tensor Model::graph_attention(const Tensor& _input, int heads, float negativeSlope) {
+  GraphAttention* op = new GraphAttention(*this, _input, heads, negativeSlope);
+  layers.push_back(op);
+  parameters.push_back(op->weight);
+  return op->outputs[0];
+}
 void Model::softmax_cross_entropy(const Tensor& logits, const Tensor& labels, const Tensor& mask) {
   layers.push_back(new SoftmaxCrossEntropy(*this, logits, labels, mask));
 }
@@ -142,6 +148,30 @@ Wiring wire(const std::vector<GnnOp*>& layers) {
 }
 template <typename T>
 T* as(GnnOp* op) { return dynamic_cast<T*>(op); }
+
+// The tensors an op's gathers read at halo rows (multi-GPU): region, data or grad twin.  Backward reads are listed
+// only when the op's backward runs.
+struct HaloRead { int region; bool grad; };
+std::vector<HaloRead> halo_reads(RuntimeImpl* rt, GnnOp* op) {
+  std::vector<HaloRead> r;
+  if (const ScatterGather* sg = as<ScatterGather>(op)) {
+    r.push_back({sg->inputs[0].region, false});
+    if (rt->t(sg->inputs[0].region).requiresGrad) {
+      // the backward gathers dOut (SUM, MAX, MIN) or D^-1 dOut (AVG); MAX / MIN also the winner ids
+      if (sg->scratch >= 0) r.push_back({sg->scratch, false});
+      else r.push_back({sg->outputs[0].region, true});
+      if (sg->argRegion >= 0) r.push_back({sg->argRegion, false});
+    }
+  } else if (const GraphAttention* ga = as<GraphAttention>(op)) {
+    // forward: h and s_src / s_dst; backward (always: the op has a parameter): dOut and lse / c.  The backward also
+    // reads h at halo rows, but those rows still hold this step's values: only the forward's exchange writes them.
+    r.push_back({ga->inputs[0].region, false});
+    r.push_back({ga->attRegion, false});
+    r.push_back({ga->outputs[0].region, true});
+    r.push_back({ga->bstRegion, false});
+  }
+  return r;
+}
 }  // namespace
 
 // gnn.cc:625-673.  No graph loading / ResourceManager creation left to do here
@@ -165,7 +195,7 @@ bool Model::init(const Config& config) {
     bool any = false;
     for (int j = 0; j < op->numInputs; j++)
       if (op->inputs[j].region >= 0) any = any || rt->t(op->inputs[j].region).requiresGrad;
-    if (as<Linear>(op)) any = true;
+    if (as<Linear>(op) || as<GraphAttention>(op)) any = true;   // ops with a parameter
     for (int j = 0; j < op->numOutputs; j++) {
       rt->t(op->outputs[j].region).requiresGrad = any;
       rt->t(op->outputs[j].region).produced = true;
@@ -198,6 +228,14 @@ bool Model::init(const Config& config) {
           ROC_FATAL("scatter_gather(AGGR_MAX / AGGR_MIN) needs the halo exchange (unset ROC_B200_HALO=0)");
       }
     }
+    if (GraphAttention* ga = as<GraphAttention>(layers[l])) {
+      const int H = (int)ga->inputs[0].dims[0];
+      maxSg = std::max(maxSg, H);
+      ROC_CHECK(roc_gat_plan_reserve(myGraph.plan, H, ga->heads));
+      // the gathers read four tensors at halo rows; the whole-matrix all-gather has one shared buffer
+      if (rt->numParts > 1 && !myGraph.halo)
+        ROC_FATAL("graph_attention needs the halo exchange (unset ROC_B200_HALO=0)");
+    }
   }
   rt->ensure_lin_ws(ws);
   if (maxSg > 0) {
@@ -205,22 +243,13 @@ bool Model::init(const Config& config) {
     if (maxArg > 0) ROC_CHECK(roc_sg_plan_reserve_arg(myGraph.plan, maxArg));
     if (rt->numParts > 1 && !myGraph.halo) rt->ensure_gather((size_t)myGraph.numNodes * (size_t)round_up4(maxSg));
     if (myGraph.halo) {
-      // the tensors a ScatterGather reads get the halo slab appended to their own rows
+      // the tensors a gather reads get the halo slab appended to their own rows.  Usually the buffer does not exist
+      // yet (lazy allocation).  A tensor the script already filled — e.g. an SGC-style scatter_gather(input) after
+      // load_features / set_tensor, which the reference's script order (gnn.cc:72-74) allows — is re-homed with the
+      // halo rows behind its own.
       rt->ensure_sendbuf((myGraph.numSendRows ? myGraph.numSendRows : 1) * (size_t)round_up4(maxSg));
-      for (size_t l = 0; l < layers.size(); l++) {
-        if (!as<ScatterGather>(layers[l])) continue;
-        TensorImpl& xin = rt->t(layers[l]->inputs[0].region);
-        TensorImpl& xout = rt->t(layers[l]->outputs[0].region);
-        // Usually neither buffer exists yet (lazy allocation).  A tensor the script already filled — e.g. an
-        // SGC-style scatter_gather(input) after load_features / set_tensor, which the reference's script order
-        // (gnn.cc:72-74) allows — is re-homed with the halo rows behind its own.
-        rt->grow_halo(xin, /*grad=*/false, myGraph.numHalo);
-        rt->grow_halo(xout, /*grad=*/true, myGraph.numHalo);
-        // AVG's backward gathers its scaled dOut rows, MAX / MIN's the winner ids: halo rows for them too
-        const ScatterGather* sg = as<ScatterGather>(layers[l]);
-        if (sg->scratch >= 0) rt->grow_halo(rt->t(sg->scratch), /*grad=*/false, myGraph.numHalo);
-        if (sg->argRegion >= 0) rt->grow_halo(rt->t(sg->argRegion), /*grad=*/false, myGraph.numHalo);
-      }
+      for (size_t l = 0; l < layers.size(); l++)
+        for (const HaloRead& r : halo_reads(rt, layers[l])) rt->grow_halo(rt->t(r.region), r.grad, myGraph.numHalo);
       // Exchange by peer writes (roc_push_rows): the slabs exist now and every partition maps the others' copies.
       // ROC_B200_HALO=nccl keeps the staged-rows + NCCL all-to-all-v exchange (cross-check; also the fallback when
       // CUDA IPC is not available between the devices).
@@ -232,21 +261,9 @@ bool Model::init(const Config& config) {
       // ROC_B200_HALO=push | ce forces one.
       rt->p2pCopyEngines = (he && he[0] == 'c') ? true : (he && he[0] == 'p') ? false : rt->numParts == 2;
       for (size_t l = 0; l < layers.size() && rt->p2p; l++) {
-        const ScatterGather* sg = as<ScatterGather>(layers[l]);
-        if (!sg) continue;
-        const int rin = layers[l]->inputs[0].region, rout = layers[l]->outputs[0].region;
-        rt->data(rin);
-        if (!rt->open_peers(rt->t(rin), false)) { rt->p2p = false; break; }
-        if (rt->t(rin).requiresGrad) {
-          // the tensor the backward gathers: dOut (SUM, MAX, MIN) or D^-1 dOut (AVG); MAX / MIN also the winner ids
-          const int rg = sg->scratch >= 0 ? sg->scratch : rout;
-          const bool isGrad = sg->scratch < 0;
-          if (isGrad) rt->grad(rg); else rt->data(rg);
-          if (!rt->open_peers(rt->t(rg), isGrad)) { rt->p2p = false; break; }
-          if (sg->argRegion >= 0) {
-            rt->data(sg->argRegion);
-            if (!rt->open_peers(rt->t(sg->argRegion), false)) { rt->p2p = false; break; }
-          }
+        for (const HaloRead& r : halo_reads(rt, layers[l])) {
+          if (r.grad) rt->grad(r.region); else rt->data(r.region);
+          if (!rt->open_peers(rt->t(r.region), r.grad)) { rt->p2p = false; break; }
         }
       }
       if (rt->myPart == 0)
@@ -355,7 +372,8 @@ bool Model::init(const Config& config) {
   for (size_t l = 0; l < layers.size(); l++) layers[l]->init(*this);
   rt->opNames.clear();
   for (size_t l = 0; l < layers.size(); l++) {
-    const char* nm = as<ScatterGather>(layers[l]) ? "scatter_gather" : as<Linear>(layers[l]) ? "linear" :
+    const char* nm = as<ScatterGather>(layers[l]) ? "scatter_gather" : as<GraphAttention>(layers[l]) ? "graph_attention" :
+                     as<Linear>(layers[l]) ? "linear" :
                      as<InDegreeNorm>(layers[l]) ? "indegree_norm" : as<Activation>(layers[l]) ? "activation" :
                      as<Dropout>(layers[l]) ? "dropout" : as<Element>(layers[l]) ? "add" :
                      as<SoftmaxCrossEntropy>(layers[l]) ? "softmax_cross_entropy" : "op";
@@ -761,6 +779,70 @@ void ScatterGather::backward(const Model& model) {
   rt->sg_begin(H);
   ROC_CHECK(roc_sg_forward_planned(model.myGraph.plan, H, src, ld, dst, rt->t(dstRegion).ld, bwdEpilogue, rt->stream));
   rt->sg_end();
+}
+
+// ------------------------------------------------------- GraphAttention -----
+GraphAttention::GraphAttention(const Model& model, const Tensor& _input, int _heads, float _slope)
+    : GnnOp(_input), heads(_heads), slope(_slope), attRegion(-1), bstRegion(-1), dsRegion(-1), work(nullptr) {
+  ROC_ASSERT(inputs[0].type == Tensor::NODE_TENSOR);
+  ROC_ASSERT(inputs[0].numDim == 2);
+  ROC_ASSERT(inputs[0].dims[1] == model.myGraph.numNodes);
+  const int H = (int)inputs[0].dims[0];
+  if (roc_gat_supported(H, heads) != ROC_OK) {
+    char b[256];
+    snprintf(b, sizeof(b), "graph_attention: unsupported shape H = %d, heads = %d (heads in {1, 2, 4, 8}, H <= 256, "
+             "H / heads a multiple of 4 when heads > 1)", H, heads);
+    ROC_FATAL(b);
+  }
+  numOutputs = 1;
+  outputs[0] = model.create_node_tensor<DATATYPE>(H);
+  weight = model.create_weight_tensor(H, 2, NULL);   // GlorotUniform; row 0 a_src, row 1 a_dst
+  // per-op buffers, allocated with the op (nothing is allocated inside a step)
+  const int A = 2 * heads;
+  attRegion = model.ctx->new_tensor(model.local_rows(), A, round_up4(A), false, false);
+  bstRegion = model.ctx->new_tensor(model.local_rows(), A, round_up4(A), false, false);
+  dsRegion = model.ctx->new_tensor(model.local_rows(), A, round_up4(A), false, false);
+  work = model.ctx->dmalloc(roc_gat_finish_workspace_bytes(H));
+}
+void GraphAttention::init(const Model&) {}
+
+void GraphAttention::forward(const Model& model) {
+  RuntimeImpl* rt = model.ctx;
+  const int H = (int)inputs[0].dims[0];
+  TensorImpl& x = rt->t(inputs[0].region);
+  TensorImpl& at = rt->t(attRegion);
+  TensorImpl& bt = rt->t(bstRegion);
+  // s_src / s_dst of the own rows, then h and them at the halo rows
+  ROC_CHECK(roc_gat_scores(model.local_rows(), H, heads, rt->data(inputs[0].region), x.ld, rt->data(weight.region),
+                           rt->data(attRegion), at.ld, rt->stream));
+  const float* h = gathered(model, rt->data(inputs[0].region), x.ld, H, &x, false);
+  const float* att = gathered(model, rt->data(attRegion), at.ld, 2 * heads, &at, false);
+  ROC_CHECK(roc_gat_forward(model.myGraph.plan, H, heads, slope, h, x.ld, att, at.ld, rt->data(bstRegion), bt.ld,
+                            rt->data(outputs[0].region), rt->t(outputs[0].region).ld, rt->stream));
+}
+
+void GraphAttention::backward(const Model& model) {
+  RuntimeImpl* rt = model.ctx;
+  ROC_ASSERT(resetInputGrads[0]);   // dh is overwritten, like ScatterGather's
+  const int H = (int)inputs[0].dims[0];
+  TensorImpl& x = rt->t(inputs[0].region);
+  TensorImpl& y = rt->t(outputs[0].region);
+  TensorImpl& at = rt->t(attRegion);
+  TensorImpl& bt = rt->t(bstRegion);
+  TensorImpl& dt = rt->t(dsRegion);
+  // c = <dOut, out> per row and head, then dOut and (lse | c) at the halo rows.  h's halo rows are the forward's:
+  // nothing rewrites them between the two passes, so they need no second exchange.
+  ROC_CHECK(roc_gat_bwd_c(model.local_rows(), H, heads, rt->grad(outputs[0].region), y.ld, rt->data(outputs[0].region),
+                          y.ld, rt->data(bstRegion), bt.ld, rt->stream));
+  const float* dOut = gathered(model, rt->grad(outputs[0].region), y.ld, H, &y, true);
+  const float* bst = gathered(model, rt->data(bstRegion), bt.ld, 2 * heads, &bt, false);
+  float* dh = rt->grad(inputs[0].region);
+  ROC_CHECK(roc_gat_backward(model.myGraph.plan, H, heads, slope, rt->data(inputs[0].region), x.ld,
+                             rt->data(attRegion), at.ld, bst, bt.ld, dOut, y.ld, dh, x.ld, rt->data(dsRegion), dt.ld,
+                             rt->stream));
+  ROC_CHECK(roc_gat_bwd_finish(model.local_rows(), H, heads, rt->data(inputs[0].region), x.ld, rt->data(weight.region),
+                               rt->data(dsRegion), dt.ld, dh, x.ld, rt->grad(weight.region), work,
+                               roc_gat_finish_workspace_bytes(H), rt->stream));
 }
 
 // --------------------------------------------------------- InDegreeNorm -----

@@ -34,6 +34,7 @@
 // Algorithmic bytes per launch (DESIGN.md): E*(4H+4) + Nloc*(4H+8).
 #include <cub/cub.cuh>
 #include <thrust/iterator/counting_iterator.h>
+#include <algorithm>
 #include <cstdlib>
 #include <cstring>
 #include <new>
@@ -1756,6 +1757,593 @@ static int ensure_carry_arg(roc_sg_plan* plan, size_t ld, cudaStream_t st, bool 
   return grow_carry(plan, plan->carryArg, plan->carryArgLd, ld, st, inStream);
 }
 
+// ------------------------------------------------------------------ graph attention (GAT) ---
+// out[v, k-block] = sum over u in in(v) of alpha[v<-u,k] h[u, k-block], alpha = softmax over the row's in-edges of
+// LeakyReLU(s_src[u,k] + s_dst[v,k]).  Per-node tensors: att[r] = (s_src[0..K) | s_dst[0..K)), bst[r] = (lse[0..K) |
+// c[0..K)), both indexed like h ([own rows | halo rows]).  Kernels, all on the plan's chunk schedule, no atomics:
+//   k_gat_rowdot        s_src / s_dst (forward) and c = <dOut, out> (backward): a warp per row, fixed-order dots
+//   k_gat_stats         lse per row and head; a thread per chunk with an online (max, Z) pair; rows cut at chunk
+//                       boundaries leave (max, Z) parts (owner: in its bst row, later chunks: in the carry slots)
+//   k_gat_stats_fixup   merges those parts in chunk order (a warp per cut row, lanes own contiguous carry blocks)
+//   sg_gat_kernel       kernel A with each gathered row scaled by alpha before the add; cut rows: SUM's fix-ups
+//   sg_gat_bwd_kernel   row u gathers dOut[v], h[v], att[v], bst[v]: dh_agg[u] and ds_src / ds_dst[u]; cut rows:
+//                       SUM's fix-ups over the [dh | ds] carry part
+//   k_gat_finish        dh += ds_src a_src + ds_dst a_dst, and the fixed-block partials of da; k_gat_da_reduce sums
+//                       the partials in block order
+// alpha is never stored: gat_alpha below is the one place it is computed, by the forward and the backward alike.
+constexpr int GAT_ROWDOT_WARPS = 8;
+constexpr int GAT_FINISH_THREADS = 256;
+constexpr uint32_t GAT_FINISH_BLOCKS = 1184;   // fixed: the da partial order depends on the row count only
+
+__device__ __forceinline__ float gat_leaky(float z, float slope) { return z > 0.f ? z : z * slope; }
+__device__ __forceinline__ float gat_dleaky(float z, float slope) { return z > 0.f ? 1.f : slope; }
+__device__ __forceinline__ float gat_alpha(float sSrcU, float sDstV, float lseV, float slope) {
+  return expf(gat_leaky(sSrcU + sDstV, slope) - lseV);
+}
+// (m, z) <- (m, z) + (m2, z2) for z = sum exp(e - m).  An empty part is (-inf, 0).
+__device__ __forceinline__ void gat_lse_merge(float& m, float& z, float m2, float z2) {
+  const float M = fmaxf(m, m2);
+  if (M == -INFINITY) return;
+  z = z * expf(m - M) + z2 * expf(m2 - M);
+  m = M;
+}
+
+// dst1[r][k] = <x[r, k-block], y1[k-block]> (y1 one vector when ldY1 == 0, else a row per r); the same for y2 when
+// given.  A warp per row, lanes stride the head's columns, xor-butterfly sum: fixed order.
+__global__ void __launch_bounds__(32 * GAT_ROWDOT_WARPS)
+k_gat_rowdot(int64_t rows, int F, int K, const float* __restrict__ x, int64_t ldX, const float* __restrict__ y1,
+             int64_t ldY1, const float* __restrict__ y2, int64_t ldY2, float* __restrict__ dst1,
+             float* __restrict__ dst2, int64_t ldD) {
+  const int64_t r = (int64_t)blockIdx.x * GAT_ROWDOT_WARPS + threadIdx.x / 32;
+  const int lane = threadIdx.x & 31;
+  if (r >= rows) return;
+  const float* xr = x + r * ldX;
+  const float* a = y1 + r * ldY1;
+  const float* b = y2 ? y2 + r * ldY2 : nullptr;
+  for (int k = 0; k < K; k++) {
+    float p1 = 0.f, p2 = 0.f;
+    for (int j = lane; j < F; j += 32) {
+      const float xv = xr[k * F + j];
+      p1 = fmaf(xv, a[k * F + j], p1);
+      if (b) p2 = fmaf(xv, b[k * F + j], p2);
+    }
+#pragma unroll
+    for (int o = 16; o >= 1; o >>= 1) {
+      p1 += __shfl_xor_sync(0xffffffffu, p1, o);
+      p2 += __shfl_xor_sync(0xffffffffu, p2, o);
+    }
+    if (lane == 0) {
+      dst1[r * ldD + k] = p1;
+      if (b) dst2[r * ldD + k] = p2;
+    }
+  }
+}
+
+struct GatParams {
+  SgParams p;               // schedule; in / out / carry as the kernel uses them (VEC-float units)
+  const float* att;         // [own | halo][ldA]  s_src | s_dst
+  const float* bst;         // [own | halo][ldB]  lse | c  (written by the stats kernels, read by the others)
+  float* bstOut;            // stats: the same rows, writable
+  const float* dOut;        // backward: [own | halo][ldG] (VEC units)
+  float* ds;                // backward: [nloc][ldDs]  ds_src | ds_dst
+  size_t ldA, ldB, ldG, ldDs;
+  uint32_t dsOff;           // backward: float offset of the ds part in a carry slot
+  int H, F, K;              // width, floats per head, heads
+  int FQ;                   // VEC-columns per head
+  int hmode;                // per-head sums: 0 one head, 1 power-of-two heads narrower than the worker, 2 general
+  float slope;
+};
+
+// lse per row and head: one thread per chunk walks the chunk's edges in order.
+template <int K>
+__global__ void __launch_bounds__(256)
+k_gat_stats(const GatParams g) {
+  constexpr uint32_t CH = SG_CH;
+  constexpr int U = 4;
+  const SgParams& p = g.p;
+  const uint32_t w = blockIdx.x * blockDim.x + threadIdx.x;
+  if (w >= p.numChunks) return;
+  const uint4 dA = __ldg(reinterpret_cast<const uint4*>(p.desc) + 2 * (size_t)w);
+  const uint4 dB = __ldg(reinterpret_cast<const uint4*>(p.desc) + 2 * (size_t)w + 1);
+  if (dB.z & 2u) return;
+  const uint32_t ce = min(w * CH + CH, p.E);
+  uint32_t cur = dA.z, curS = dA.w, curT = dB.x;
+  const uint32_t ee = dA.y, r1 = dB.y, carrySlot = dB.w;
+  int kind = (dB.z & 1u) ? 0 : ((curT - curS > CH) ? 2 : 1);
+  uint32_t segEnd = (kind == 1) ? curT : min(curT, ce);
+  float sd[K], m[K], z[K];
+  auto rowvals = [&]() {
+#pragma unroll
+    for (int k = 0; k < K; k++) { sd[k] = g.att[(size_t)cur * g.ldA + K + k]; m[k] = -INFINITY; z[k] = 0.f; }
+  };
+  auto flush = [&]() {
+    if (kind == 1) {
+#pragma unroll
+      for (int k = 0; k < K; k++) g.bstOut[(size_t)cur * g.ldB + k] = (curT > curS) ? m[k] + logf(z[k]) : 0.f;
+    } else {
+      // a raw (max, Z) part: the owner's in its own bst row (its c columns are free in the forward), later
+      // chunks' in their carry slot
+      float* d = (kind == 2) ? g.bstOut + (size_t)cur * g.ldB : static_cast<float*>(p.carry) + (size_t)carrySlot * p.ldC;
+#pragma unroll
+      for (int k = 0; k < K; k++) { d[k] = m[k]; d[K + k] = z[k]; }
+    }
+  };
+  auto advance = [&]() {
+    cur += 1; curS = curT; curT = p.rs[cur + 1];
+    const bool heavy = curT - curS > CH;
+    segEnd = heavy ? min(curT, ce) : curT;
+    kind = heavy ? 2 : 1;
+    rowvals();
+  };
+  rowvals();
+  const uint32_t eLast = ee - 1u;
+#pragma unroll 1
+  for (uint32_t base = dA.x; base < ee; base += U) {
+    float ss[U][K];
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+      const uint32_t src = __ldg(p.col + min(base + (uint32_t)u, eLast));
+#pragma unroll
+      for (int k = 0; k < K; k++) ss[u][k] = __ldg(g.att + (size_t)src * g.ldA + k);
+    }
+#pragma unroll
+    for (int u = 0; u < U; u++) {
+      const uint32_t e = base + (uint32_t)u;
+      if (e < ee) {
+        while (e == segEnd) { flush(); advance(); }
+#pragma unroll
+        for (int k = 0; k < K; k++) gat_lse_merge(m[k], z[k], gat_leaky(ss[u][k] + sd[k], g.slope), 1.f);
+      }
+    }
+  }
+  flush();
+  while (cur + 1 < r1) { advance(); flush(); }   // trailing zero-degree rows
+}
+
+// Rows cut at chunk boundaries (heavy and big alike): a warp per row; lane l merges the l-th contiguous block of the
+// carry parts, lane 0 then merges owner + blocks in lane order.
+template <int K>
+__global__ void __launch_bounds__(256)
+k_gat_stats_fixup(const GatParams g) {
+  constexpr uint32_t CH = SG_CH;
+  const SgParams& p = g.p;
+  const uint32_t wg = (blockIdx.x * blockDim.x + threadIdx.x) / 32;
+  const int lane = threadIdx.x & 31;
+  if (wg >= p.numHeavy + p.numBig) return;
+  const uint32_t R = wg < p.numHeavy ? p.heavyRows[wg] : p.bigRows[wg - p.numHeavy];
+  const uint32_t s = p.rs[R], t = p.rs[R + 1];
+  const uint32_t n = (t - 1) / CH - s / CH;
+  const uint32_t slot0 = p.carryIdx[s / CH + 1];
+  const uint32_t per = (n + 31) / 32;
+  const uint32_t k0 = min(n, (uint32_t)lane * per), k1 = min(n, k0 + per);
+  const float* cv = static_cast<const float*>(p.carry);
+  float m[K], z[K];
+#pragma unroll
+  for (int k = 0; k < K; k++) { m[k] = -INFINITY; z[k] = 0.f; }
+  for (uint32_t c = k0; c < k1; c++) {
+    const float* part = cv + (size_t)(slot0 + c) * p.ldC;
+#pragma unroll
+    for (int k = 0; k < K; k++) gat_lse_merge(m[k], z[k], part[k], part[K + k]);
+  }
+  float* row = g.bstOut + (size_t)R * g.ldB;
+  float om[K], oz[K];
+#pragma unroll
+  for (int k = 0; k < K; k++) { om[k] = row[k]; oz[k] = row[K + k]; }
+  for (int l = 0; l < 32; l++) {
+#pragma unroll
+    for (int k = 0; k < K; k++) {
+      const float mm = __shfl_sync(0xffffffffu, m[k], l), zz = __shfl_sync(0xffffffffu, z[k], l);
+      gat_lse_merge(om[k], oz[k], mm, zz);
+    }
+  }
+  if (lane == 0) {
+#pragma unroll
+    for (int k = 0; k < K; k++) { row[k] = om[k] + logf(oz[k]); row[K + k] = 0.f; }
+  }
+}
+
+// Per-head sums of per-lane partials p[ch] (lane's VEC-column lane + ch * L lies in head hd[ch]) over the worker's
+// L lanes; every lane ends with its heads' sums, bitwise equal across the lanes (xor butterflies).
+template <int L, int NCH>
+__device__ __forceinline__ void gat_headsum(float (&p)[NCH], const int (&hd)[NCH], const GatParams& g, unsigned wmask) {
+  if (g.hmode == 0) {
+    float s = 0.f;
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) s += p[ch];
+#pragma unroll
+    for (int o = L / 2; o >= 1; o >>= 1) s += __shfl_xor_sync(wmask, s, o);
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) p[ch] = s;
+  } else if (g.hmode == 1) {
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++)
+      for (int o = g.FQ / 2; o >= 1; o >>= 1) p[ch] += __shfl_xor_sync(wmask, p[ch], o);
+  } else {
+    float q[NCH];
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) q[ch] = 0.f;
+    for (int k = 0; k < g.K; k++) {
+      float s = 0.f;
+#pragma unroll
+      for (int ch = 0; ch < NCH; ch++) s += (hd[ch] == k) ? p[ch] : 0.f;
+#pragma unroll
+      for (int o = L / 2; o >= 1; o >>= 1) s += __shfl_xor_sync(wmask, s, o);
+#pragma unroll
+      for (int ch = 0; ch < NCH; ch++) if (hd[ch] == k) q[ch] = s;
+    }
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) p[ch] = q[ch];
+  }
+}
+
+// Weighted aggregate: kernel A's schedule and per-row order, each gathered row scaled by its alpha (per head) before
+// the add.  Rows cut at chunk boundaries store raw partial sums; SUM's fix-up kernels finish them (epi = 0).
+template <int VEC, int L, int NCH, int U, int MINB>
+__global__ void __launch_bounds__(SG_THREADS, MINB)
+sg_gat_kernel(const GatParams g) {
+  constexpr int WPB = SG_THREADS / L;
+  constexpr uint32_t CH = SG_CH;
+  const SgParams& p = g.p;
+  const int lane = threadIdx.x % L;
+  const uint32_t w = blockIdx.x * WPB + threadIdx.x / L;
+  if (w >= p.numChunks) return;
+  bool act[NCH];
+  int hd[NCH];
+#pragma unroll
+  for (int ch = 0; ch < NCH; ch++) {
+    act[ch] = (uint32_t)(lane + ch * L) < p.Q;
+    hd[ch] = min((uint32_t)(lane + ch * L), p.Q - 1u) / (uint32_t)g.FQ;
+  }
+  const uint32_t ce = min(w * CH + CH, p.E);
+  const uint4 dA = __ldg(reinterpret_cast<const uint4*>(p.desc) + 2 * (size_t)w);
+  const uint4 dB = __ldg(reinterpret_cast<const uint4*>(p.desc) + 2 * (size_t)w + 1);
+  if (dB.z & 2u) return;
+  uint32_t cur = dA.z, curS = dA.w, curT = dB.x;
+  const uint32_t e = dA.x, ee = dA.y, r1 = dB.y, carrySlot = dB.w;
+  int kind = (dB.z & 1u) ? 0 : ((curT - curS > CH) ? 2 : 1);
+  uint32_t segEnd = (kind == 1) ? curT : min(curT, ce);
+
+  float acc[NCH][VEC], sd[NCH], ls[NCH];
+#pragma unroll
+  for (int ch = 0; ch < NCH; ch++)
+#pragma unroll
+    for (int k = 0; k < VEC; k++) acc[ch][k] = 0.f;
+  auto rowvals = [&]() {
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) {
+      sd[ch] = g.att[(size_t)cur * g.ldA + g.K + hd[ch]];
+      ls[ch] = g.bst[(size_t)cur * g.ldB + hd[ch]];
+    }
+  };
+  auto flush = [&]() {
+    float* dst = (kind == 0) ? static_cast<float*>(p.carry) + (size_t)carrySlot * p.ldC * VEC
+                             : static_cast<float*>(p.out) + (size_t)cur * p.ldOut * VEC;
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) {
+      if (act[ch]) stv<VEC>(dst + (lane + ch * L) * VEC, acc[ch]);
+#pragma unroll
+      for (int k = 0; k < VEC; k++) acc[ch][k] = 0.f;
+    }
+  };
+  auto advance = [&]() {
+    cur += 1; curS = curT; curT = p.rs[cur + 1];
+    const bool heavy = curT - curS > CH;
+    segEnd = heavy ? min(curT, ce) : curT;
+    kind = heavy ? 2 : 1;
+    rowvals();
+  };
+  rowvals();
+  const float* inl[NCH];
+#pragma unroll
+  for (int ch = 0; ch < NCH; ch++) inl[ch] = static_cast<const float*>(p.in) + min((uint32_t)(lane + ch * L), p.Q - 1u) * VEC;
+  const uint64_t ldInF = (uint64_t)p.ldIn * VEC;
+  const uint32_t eLast = ee - 1u;
+#pragma unroll 1
+  for (uint32_t base = e; base < ee; base += U) {
+    const uint32_t cnt = min((uint32_t)U, ee - base);
+    uint32_t srcs[U];
+#pragma unroll
+    for (int u = 0; u < U; u++) srcs[u] = __ldg(p.col + min(base + (uint32_t)u, eLast));
+    float v[U][NCH][VEC], ss[U][NCH];
+#pragma unroll
+    for (int u = 0; u < U; u++)
+#pragma unroll
+      for (int ch = 0; ch < NCH; ch++) {
+        ldv_nc<VEC>(v[u][ch], inl[ch] + srcs[u] * ldInF);
+        ss[u][ch] = __ldg(g.att + (size_t)srcs[u] * g.ldA + hd[ch]);
+      }
+    uint32_t pos = 0;
+    for (;;) {
+      const uint32_t lim = min(cnt, segEnd - base);
+#pragma unroll
+      for (int u = 0; u < U; u++) {
+        if ((uint32_t)u >= pos && (uint32_t)u < lim) {
+#pragma unroll
+          for (int ch = 0; ch < NCH; ch++) {
+            const float a = gat_alpha(ss[u][ch], sd[ch], ls[ch], g.slope);
+#pragma unroll
+            for (int k = 0; k < VEC; k++) acc[ch][k] = fmaf(a, v[u][ch][k], acc[ch][k]);
+          }
+        }
+      }
+      pos = lim;
+      if (pos >= cnt) break;
+      flush();
+      advance();
+    }
+  }
+  flush();
+  while (cur + 1 < r1) { advance(); flush(); }
+}
+
+// Backward gather: row u (the plan's row) walks its in-edges v (by the CSR's symmetry, the v that u feeds):
+//   dh_agg[u] += alpha[v<-u] dOut[v]
+//   ds_src[u] += alpha[v<-u] (<dOut[v], h[u]> - c[v]) LeakyReLU'(s_src[u] + s_dst[v])
+//   ds_dst[u] += alpha[u<-v] (<dOut[u], h[v]> - c[u]) LeakyReLU'(s_src[v] + s_dst[u])
+// (per head).  Two rows gathered per edge.  Rows cut at chunk boundaries: the owner stores its raw parts into the
+// dh and ds rows, later chunks into the carry slot ([dh | ds] at dsOff); SUM's fix-ups sum them in chunk order.
+template <int VEC, int L, int NCH, int U, int MINB>
+__global__ void __launch_bounds__(SG_THREADS, MINB)
+sg_gat_bwd_kernel(const GatParams g) {
+  constexpr int WPB = SG_THREADS / L;
+  constexpr uint32_t CH = SG_CH;
+  const SgParams& p = g.p;
+  const int lane = threadIdx.x % L;
+  const uint32_t w = blockIdx.x * WPB + threadIdx.x / L;
+  if (w >= p.numChunks) return;
+  const unsigned wmask = (L == 32) ? 0xffffffffu : (((1u << L) - 1u) << (((threadIdx.x & 31) / L) * L));
+  bool act[NCH], first[NCH];
+  int hd[NCH];
+#pragma unroll
+  for (int ch = 0; ch < NCH; ch++) {
+    const uint32_t t = lane + ch * L;
+    act[ch] = t < p.Q;
+    hd[ch] = min(t, p.Q - 1u) / (uint32_t)g.FQ;
+    first[ch] = act[ch] && (t % (uint32_t)g.FQ) == 0;
+  }
+  // a lane's real columns: pad and clamped columns enter no dot
+  auto real = [&](int ch, int k) { return (int)((lane + ch * L) * VEC + k) < g.H; };
+  const uint32_t ce = min(w * CH + CH, p.E);
+  const uint4 dA = __ldg(reinterpret_cast<const uint4*>(p.desc) + 2 * (size_t)w);
+  const uint4 dB = __ldg(reinterpret_cast<const uint4*>(p.desc) + 2 * (size_t)w + 1);
+  if (dB.z & 2u) return;
+  uint32_t cur = dA.z, curS = dA.w, curT = dB.x;
+  const uint32_t e = dA.x, ee = dA.y, r1 = dB.y, carrySlot = dB.w;
+  int kind = (dB.z & 1u) ? 0 : ((curT - curS > CH) ? 2 : 1);
+  uint32_t segEnd = (kind == 1) ? curT : min(curT, ce);
+
+  const float* hIn = static_cast<const float*>(p.in);
+  const uint64_t ldHF = (uint64_t)p.ldIn * VEC, ldGF = (uint64_t)g.ldG * VEC;
+  uint32_t cofs[NCH];
+#pragma unroll
+  for (int ch = 0; ch < NCH; ch++) cofs[ch] = min((uint32_t)(lane + ch * L), p.Q - 1u) * VEC;
+
+  float acc[NCH][VEC], dss[NCH], dsd[NCH];
+  float gu[NCH][VEC], hu[NCH][VEC], ssu[NCH], sdu[NCH], lsu[NCH], cu[NCH];
+  auto zero = [&]() {
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) {
+      dss[ch] = 0.f; dsd[ch] = 0.f;
+#pragma unroll
+      for (int k = 0; k < VEC; k++) acc[ch][k] = 0.f;
+    }
+  };
+  auto rowvals = [&]() {
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) {
+      ldv<VEC>(gu[ch], g.dOut + (uint64_t)cur * ldGF + cofs[ch]);
+      ldv<VEC>(hu[ch], hIn + (uint64_t)cur * ldHF + cofs[ch]);
+      ssu[ch] = g.att[(size_t)cur * g.ldA + hd[ch]];
+      sdu[ch] = g.att[(size_t)cur * g.ldA + g.K + hd[ch]];
+      lsu[ch] = g.bst[(size_t)cur * g.ldB + hd[ch]];
+      cu[ch] = g.bst[(size_t)cur * g.ldB + g.K + hd[ch]];
+    }
+  };
+  auto flush = [&]() {
+    float* dst = (kind == 0) ? static_cast<float*>(p.carry) + (size_t)carrySlot * p.ldC * VEC
+                             : static_cast<float*>(p.out) + (size_t)cur * p.ldOut * VEC;
+    float* dsd_ = (kind == 0) ? static_cast<float*>(p.carry) + (size_t)carrySlot * p.ldC * VEC + g.dsOff
+                              : g.ds + (size_t)cur * g.ldDs;
+#pragma unroll
+    for (int ch = 0; ch < NCH; ch++) {
+      if (act[ch]) stv<VEC>(dst + (lane + ch * L) * VEC, acc[ch]);
+      if (first[ch]) { dsd_[hd[ch]] = dss[ch]; dsd_[g.K + hd[ch]] = dsd[ch]; }
+    }
+    zero();
+  };
+  auto advance = [&]() {
+    cur += 1; curS = curT; curT = p.rs[cur + 1];
+    const bool heavy = curT - curS > CH;
+    segEnd = heavy ? min(curT, ce) : curT;
+    kind = heavy ? 2 : 1;
+    rowvals();
+  };
+  zero();
+  rowvals();
+  const uint32_t eLast = ee - 1u;
+#pragma unroll 1
+  for (uint32_t base = e; base < ee; base += U) {
+    const uint32_t cnt = min((uint32_t)U, ee - base);
+    uint32_t srcs[U];
+#pragma unroll
+    for (int u = 0; u < U; u++) srcs[u] = __ldg(p.col + min(base + (uint32_t)u, eLast));
+    float gv[U][NCH][VEC], hv[U][NCH][VEC], ssv[U][NCH], sdv[U][NCH], lsv[U][NCH], cvv[U][NCH];
+#pragma unroll
+    for (int u = 0; u < U; u++)
+#pragma unroll
+      for (int ch = 0; ch < NCH; ch++) {
+        ldv_nc<VEC>(gv[u][ch], g.dOut + srcs[u] * ldGF + cofs[ch]);
+        ldv_nc<VEC>(hv[u][ch], hIn + srcs[u] * ldHF + cofs[ch]);
+        const float* at = g.att + (size_t)srcs[u] * g.ldA;
+        const float* bt = g.bst + (size_t)srcs[u] * g.ldB;
+        ssv[u][ch] = __ldg(at + hd[ch]); sdv[u][ch] = __ldg(at + g.K + hd[ch]);
+        lsv[u][ch] = __ldg(bt + hd[ch]); cvv[u][ch] = __ldg(bt + g.K + hd[ch]);
+      }
+    uint32_t pos = 0;
+    for (;;) {
+      const uint32_t lim = min(cnt, segEnd - base);
+#pragma unroll
+      for (int u = 0; u < U; u++) {
+        if ((uint32_t)u >= pos && (uint32_t)u < lim) {
+          float d1[NCH], d2[NCH];
+#pragma unroll
+          for (int ch = 0; ch < NCH; ch++) {
+            float a = 0.f, b = 0.f;
+#pragma unroll
+            for (int k = 0; k < VEC; k++) {
+              if (real(ch, k)) {
+                a = fmaf(gv[u][ch][k], hu[ch][k], a);
+                b = fmaf(gu[ch][k], hv[u][ch][k], b);
+              }
+            }
+            d1[ch] = a; d2[ch] = b;
+          }
+          gat_headsum<L, NCH>(d1, hd, g, wmask);
+          gat_headsum<L, NCH>(d2, hd, g, wmask);
+#pragma unroll
+          for (int ch = 0; ch < NCH; ch++) {
+            const float z1 = ssu[ch] + sdv[u][ch];
+            const float a1 = gat_alpha(ssu[ch], sdv[u][ch], lsv[u][ch], g.slope);
+#pragma unroll
+            for (int k = 0; k < VEC; k++) acc[ch][k] = fmaf(a1, gv[u][ch][k], acc[ch][k]);
+            dss[ch] = fmaf(a1 * (d1[ch] - cvv[u][ch]), gat_dleaky(z1, g.slope), dss[ch]);
+            const float z2 = ssv[u][ch] + sdu[ch];
+            const float a2 = gat_alpha(ssv[u][ch], sdu[ch], lsu[ch], g.slope);
+            dsd[ch] = fmaf(a2 * (d2[ch] - cu[ch]), gat_dleaky(z2, g.slope), dsd[ch]);
+          }
+        }
+      }
+      pos = lim;
+      if (pos >= cnt) break;
+      flush();
+      advance();
+    }
+  }
+  flush();
+  while (cur + 1 < r1) { advance(); flush(); }
+}
+
+// dh[r][j] += ds_src[r][hd(j)] a_src[j] + ds_dst[r][hd(j)] a_dst[j], and block b's partial of
+// da_src[j] = sum_r ds_src[r][hd(j)] h[r][j] (da_dst alike) over its fixed row range, rows in order.
+__global__ void __launch_bounds__(GAT_FINISH_THREADS)
+k_gat_finish(int64_t rows, int H, int F, int K, const float* __restrict__ h, int64_t ldH, const float* __restrict__ a,
+             const float* __restrict__ ds, int64_t ldDs, float* __restrict__ dh, int64_t ldDh, float* __restrict__ part) {
+  __shared__ float red[GAT_FINISH_THREADS * 2];
+  const int S = GAT_FINISH_THREADS / H;                 // row lanes per block
+  const int j = threadIdx.x % H, sub = threadIdx.x / H;
+  const int64_t per = (rows + gridDim.x - 1) / gridDim.x;
+  const int64_t r0 = min(rows, (int64_t)blockIdx.x * per), r1 = min(rows, r0 + per);
+  float s1 = 0.f, s2 = 0.f;
+  if (sub < S) {
+    const int k = j / F;
+    const float as = a[j], ad = a[H + j];
+#pragma unroll 4
+    for (int64_t r = r0 + sub; r < r1; r += S) {
+      const float x = h[r * ldH + j], g1 = ds[r * ldDs + k], g2 = ds[r * ldDs + K + k];
+      float* d = dh + r * ldDh + j;
+      *d = fmaf(g2, ad, fmaf(g1, as, *d));
+      s1 = fmaf(g1, x, s1);
+      s2 = fmaf(g2, x, s2);
+    }
+  }
+  red[threadIdx.x] = s1;
+  red[GAT_FINISH_THREADS + threadIdx.x] = s2;
+  __syncthreads();
+  if (sub == 0) {
+    float t1 = 0.f, t2 = 0.f;
+    for (int q = 0; q < S; q++) { t1 += red[q * H + j]; t2 += red[GAT_FINISH_THREADS + q * H + j]; }
+    part[(size_t)blockIdx.x * 2 * H + j] = t1;
+    part[(size_t)blockIdx.x * 2 * H + H + j] = t2;
+  }
+}
+__global__ void k_gat_da_reduce(int H, uint32_t nb, const float* __restrict__ part, float* __restrict__ da) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= 2 * H) return;
+  float s = 0.f;
+  for (uint32_t b = 0; b < nb; b++) s += part[(size_t)b * 2 * H + i];
+  da[i] = s;
+}
+
+enum { GAT_FWD = 0, GAT_BWD = 1 };
+
+template <int OP, int VEC, int L, int NCH, int U, int MINB>
+static int launch_gat_cfg(const GatParams& g, cudaStream_t st) {
+  constexpr int WPB = SG_THREADS / L;
+  constexpr int UU = (OP == GAT_BWD && U > 1) ? U / 2 : U;   // two rows per edge: half the edges in flight
+  // the backward also holds its own row's dOut, h and per-node values: fewer CTAs per SM, no spills
+  constexpr int MB = (OP == GAT_BWD) ? (NCH == 1 ? 2 : 1) : MINB;
+  const SgParams& p = g.p;
+  if (p.numChunks) {
+    if constexpr (OP == GAT_FWD) sg_gat_kernel<VEC, L, NCH, UU, MINB><<<(p.numChunks + WPB - 1) / WPB, SG_THREADS, 0, st>>>(g);
+    else sg_gat_bwd_kernel<VEC, L, NCH, UU, MB><<<(p.numChunks + WPB - 1) / WPB, SG_THREADS, 0, st>>>(g);
+    ROC_LAUNCH_CHECK();
+  }
+  // cut rows are plain sums: SUM's fix-up kernels (the instantiations SUM launches) finish them
+  if (p.numHeavy) {
+    sg_fixup_kernel<VEC, L, NCH, U><<<(p.numHeavy + WPB - 1) / WPB, SG_THREADS, 0, st>>>(p);
+    ROC_LAUNCH_CHECK();
+  }
+  if (p.numBig) {
+    sg_fixup_big_kernel<VEC, L, NCH, U><<<p.numBig, SG_THREADS, 0, st>>>(p);
+    ROC_LAUNCH_CHECK();
+  }
+  return ROC_OK;
+}
+
+template <int OP, int VEC>
+static int dispatch_gat(const GatParams& g, cudaStream_t st) {
+  const uint32_t Q = g.p.Q;
+  if (Q <= 4) return launch_gat_cfg<OP, VEC, 4, 1, 4, 4>(g, st);
+  if (Q <= 8) return launch_gat_cfg<OP, VEC, 8, 1, 8, 3>(g, st);
+  if (Q <= 16) return launch_gat_cfg<OP, VEC, 16, 1, 8, 3>(g, st);
+  if (Q <= 32) return launch_gat_cfg<OP, VEC, 32, 1, 8, 3>(g, st);
+  if constexpr (VEC == 4) {
+    if (Q <= 64) return launch_gat_cfg<OP, VEC, 32, 2, 4, 2>(g, st);
+  } else {
+    if (Q <= 64) return launch_gat_cfg<OP, VEC, 32, 2, 4, 2>(g, st);
+    if (Q <= 128) return launch_gat_cfg<OP, VEC, 32, 4, 2, 2>(g, st);
+    if (Q <= 256) return launch_gat_cfg<OP, VEC, 32, 8, 1, 1>(g, st);
+  }
+  return ROC_ERR_UNSUPPORTED;
+}
+
+// the ds rows' fix-up: SUM's per-worker / per-CTA kernels on the 2K-float ds part of the carry slots
+static int gat_ds_fixup(const SgParams& p, cudaStream_t st) {
+  if (p.Q <= 4) {
+    if (p.numHeavy) { sg_fixup_kernel<1, 4, 1, 4><<<(p.numHeavy + 63) / 64, SG_THREADS, 0, st>>>(p); ROC_LAUNCH_CHECK(); }
+    if (p.numBig) { sg_fixup_big_kernel<1, 4, 1, 4><<<p.numBig, SG_THREADS, 0, st>>>(p); ROC_LAUNCH_CHECK(); }
+  } else if (p.Q <= 8) {
+    if (p.numHeavy) { sg_fixup_kernel<1, 8, 1, 8><<<(p.numHeavy + 31) / 32, SG_THREADS, 0, st>>>(p); ROC_LAUNCH_CHECK(); }
+    if (p.numBig) { sg_fixup_big_kernel<1, 8, 1, 8><<<p.numBig, SG_THREADS, 0, st>>>(p); ROC_LAUNCH_CHECK(); }
+  } else {
+    if (p.numHeavy) { sg_fixup_kernel<1, 16, 1, 8><<<(p.numHeavy + 15) / 16, SG_THREADS, 0, st>>>(p); ROC_LAUNCH_CHECK(); }
+    if (p.numBig) { sg_fixup_big_kernel<1, 16, 1, 8><<<p.numBig, SG_THREADS, 0, st>>>(p); ROC_LAUNCH_CHECK(); }
+  }
+  return ROC_OK;
+}
+
+static bool gat_shape_ok(int H, int K) {
+  if (H <= 0 || H > 256 || !(K == 1 || K == 2 || K == 4 || K == 8)) return false;
+  return K == 1 || (H % K == 0 && (H / K) % 4 == 0);
+}
+// carry slot of the widest GAT pass: the backward's [dh | ds]
+static size_t gat_carry_ld(int H, int K) { return ((size_t)H + 3) / 4 * 4 + ((size_t)2 * K + 3) / 4 * 4; }
+
+static void gat_schedule(const roc_sg_plan* pl, SgParams& p) {
+  memset(&p, 0, sizeof(p));
+  p.rs = pl->rs; p.firstRow = pl->firstRow; p.carryIdx = pl->carryIdx; p.heavyRows = pl->heavyRows; p.bigRows = pl->bigRows;
+  p.col = pl->col; p.carry = pl->carry; p.E = pl->E; p.numChunks = pl->numChunks; p.numHeavy = pl->numHeavy;
+  p.numBig = pl->numBig; p.epi = 0; p.desc = pl->desc; p.nloc = pl->nloc;
+}
+// head layout of a launch: Q VEC-columns, FQ per head; hmode as gat_headsum reads it
+static void gat_heads(GatParams& g, int H, int K, int VEC, int L) {
+  g.H = H; g.K = K; g.F = H / K;
+  g.FQ = K == 1 ? (int)g.p.Q : g.F / VEC;
+  const bool pow2 = (g.FQ & (g.FQ - 1)) == 0;
+  g.hmode = K == 1 ? 0 : (pow2 && g.FQ < L) ? 1 : 2;
+}
+static int gat_lanes(uint32_t Q) { return Q <= 4 ? 4 : Q <= 8 ? 8 : Q <= 16 ? 16 : 32; }
+
 }  // namespace roc
 
 using namespace roc;
@@ -2011,4 +2599,137 @@ extern "C" int roc_sg_backward(roc_vid_t rowLeft, roc_vid_t rowRight, roc_eid_t 
                                float* inGrad, roc_stream_t stream) {
   // Forward and backward do exactly the same thing (scattergather_kernel.cu:168-169).
   return roc_sg_forward(rowLeft, rowRight, colLeft, H, rowEnd, colSrc, outGrad, inGrad, stream);
+}
+
+// ------------------------------------------------------------------ graph attention: C ABI ---
+extern "C" int roc_gat_supported(int H, int heads) { return gat_shape_ok(H, heads) ? ROC_OK : ROC_ERR_UNSUPPORTED; }
+
+extern "C" int roc_gat_plan_reserve(roc_sg_plan* pl, int H, int heads) {
+  if (!pl) return ROC_ERR_INVALID;
+  if (!gat_shape_ok(H, heads)) return ROC_ERR_UNSUPPORTED;
+  return ensure_carry(pl, gat_carry_ld(H, heads), nullptr, false);
+}
+
+static int gat_rowdot(int64_t rows, int H, int K, const float* x, int64_t ldX, const float* y1, int64_t ldY1,
+                      const float* y2, int64_t ldY2, float* d1, float* d2, int64_t ldD, cudaStream_t st) {
+  if (rows <= 0) return ROC_OK;
+  const int64_t grid = (rows + GAT_ROWDOT_WARPS - 1) / GAT_ROWDOT_WARPS;
+  k_gat_rowdot<<<(unsigned)grid, 32 * GAT_ROWDOT_WARPS, 0, st>>>(rows, H / K, K, x, ldX, y1, ldY1, y2, ldY2, d1, d2, ldD);
+  ROC_LAUNCH_CHECK();
+  return ROC_OK;
+}
+
+extern "C" int roc_gat_scores(int64_t rows, int H, int heads, const float* h, int64_t ldH, const float* attW,
+                              float* att, int64_t ldAtt, roc_stream_t stream) {
+  if (rows < 0 || !h || !attW || !att || ldH < H || ldAtt < 2 * heads) return ROC_ERR_INVALID;
+  if (!gat_shape_ok(H, heads)) return ROC_ERR_UNSUPPORTED;
+  return gat_rowdot(rows, H, heads, h, ldH, attW, 0, attW + H, 0, att, att + heads, ldAtt, as_stream(stream));
+}
+
+extern "C" int roc_gat_bwd_c(int64_t rows, int H, int heads, const float* outGrad, int64_t ldG, const float* out,
+                             int64_t ldOut, float* bst, int64_t ldB, roc_stream_t stream) {
+  if (rows < 0 || !outGrad || !out || !bst || ldG < H || ldOut < H || ldB < 2 * heads) return ROC_ERR_INVALID;
+  if (!gat_shape_ok(H, heads)) return ROC_ERR_UNSUPPORTED;
+  return gat_rowdot(rows, H, heads, outGrad, ldG, out, ldOut, nullptr, 0, bst + heads, nullptr, ldB, as_stream(stream));
+}
+
+extern "C" int roc_gat_forward(const roc_sg_plan* plc, int H, int heads, float slope, const float* h, int64_t ldH,
+                               const float* att, int64_t ldAtt, float* bst, int64_t ldB, float* out, int64_t ldOut,
+                               roc_stream_t stream) {
+  roc_sg_plan* pl = const_cast<roc_sg_plan*>(plc);
+  if (!pl || !h || !att || !bst || !out || ldH < H || ldOut < H || ldAtt < 2 * heads || ldB < 2 * heads)
+    return ROC_ERR_INVALID;
+  if (!gat_shape_ok(H, heads)) return ROC_ERR_UNSUPPORTED;
+  cudaStream_t st = as_stream(stream);
+  int rc = ensure_carry(pl, gat_carry_ld(H, heads), st, true);
+  if (rc != ROC_OK) return rc;
+  const bool vec = (ldH % 4 == 0) && (ldOut % 4 == 0) && aligned16(h) && aligned16(out);
+  GatParams g;
+  memset(&g, 0, sizeof(g));
+  gat_schedule(pl, g.p);
+  g.p.in = h; g.p.out = out;
+  g.att = att; g.bst = bst; g.bstOut = bst; g.ldA = (size_t)ldAtt; g.ldB = (size_t)ldB; g.slope = slope;
+  g.K = heads;
+  // pass 1: lse (carries: raw (max, Z) parts of 2K floats)
+  g.p.ldC = pl->carryLd;
+  if (pl->numChunks) {
+    const unsigned grid = (pl->numChunks + 255) / 256;
+    switch (heads) {
+      case 1: k_gat_stats<1><<<grid, 256, 0, st>>>(g); break;
+      case 2: k_gat_stats<2><<<grid, 256, 0, st>>>(g); break;
+      case 4: k_gat_stats<4><<<grid, 256, 0, st>>>(g); break;
+      default: k_gat_stats<8><<<grid, 256, 0, st>>>(g); break;
+    }
+    ROC_LAUNCH_CHECK();
+  }
+  if (pl->numHeavy + pl->numBig) {
+    const unsigned grid = (pl->numHeavy + pl->numBig + 7) / 8;
+    switch (heads) {
+      case 1: k_gat_stats_fixup<1><<<grid, 256, 0, st>>>(g); break;
+      case 2: k_gat_stats_fixup<2><<<grid, 256, 0, st>>>(g); break;
+      case 4: k_gat_stats_fixup<4><<<grid, 256, 0, st>>>(g); break;
+      default: k_gat_stats_fixup<8><<<grid, 256, 0, st>>>(g); break;
+    }
+    ROC_LAUNCH_CHECK();
+  }
+  // pass 2: the weighted aggregate
+  const int VEC = vec ? 4 : 1;
+  g.p.ldIn = (size_t)ldH / VEC; g.p.ldOut = (size_t)ldOut / VEC; g.p.ldC = pl->carryLd / VEC;
+  g.p.Q = ((uint32_t)H + VEC - 1) / VEC;
+  gat_heads(g, H, heads, VEC, gat_lanes(g.p.Q));
+  return vec ? dispatch_gat<GAT_FWD, 4>(g, st) : dispatch_gat<GAT_FWD, 1>(g, st);
+}
+
+extern "C" int roc_gat_backward(const roc_sg_plan* plc, int H, int heads, float slope, const float* h, int64_t ldH,
+                                const float* att, int64_t ldAtt, const float* bst, int64_t ldB, const float* outGrad,
+                                int64_t ldG, float* inGrad, int64_t ldIn, float* ds, int64_t ldDs,
+                                roc_stream_t stream) {
+  roc_sg_plan* pl = const_cast<roc_sg_plan*>(plc);
+  if (!pl || !h || !att || !bst || !outGrad || !inGrad || !ds || ldH < H || ldG < H || ldIn < H ||
+      ldAtt < 2 * heads || ldB < 2 * heads || ldDs < 2 * heads)
+    return ROC_ERR_INVALID;
+  if (!gat_shape_ok(H, heads)) return ROC_ERR_UNSUPPORTED;
+  cudaStream_t st = as_stream(stream);
+  int rc = ensure_carry(pl, gat_carry_ld(H, heads), st, true);
+  if (rc != ROC_OK) return rc;
+  const bool vec = (ldH % 4 == 0) && (ldG % 4 == 0) && (ldIn % 4 == 0) && aligned16(h) && aligned16(outGrad) &&
+                   aligned16(inGrad);
+  const int VEC = vec ? 4 : 1;
+  GatParams g;
+  memset(&g, 0, sizeof(g));
+  gat_schedule(pl, g.p);
+  g.p.in = h; g.p.out = inGrad;
+  g.p.ldIn = (size_t)ldH / VEC; g.p.ldOut = (size_t)ldIn / VEC; g.p.ldC = pl->carryLd / VEC;
+  g.p.Q = ((uint32_t)H + VEC - 1) / VEC;
+  g.att = att; g.bst = bst; g.dOut = outGrad; g.ds = ds;
+  g.ldA = (size_t)ldAtt; g.ldB = (size_t)ldB; g.ldG = (size_t)ldG / VEC; g.ldDs = (size_t)ldDs;
+  g.dsOff = (uint32_t)(((size_t)H + 3) / 4 * 4);
+  g.slope = slope;
+  gat_heads(g, H, heads, VEC, gat_lanes(g.p.Q));
+  rc = vec ? dispatch_gat<GAT_BWD, 4>(g, st) : dispatch_gat<GAT_BWD, 1>(g, st);
+  if (rc != ROC_OK) return rc;
+  // the ds rows of cut rows: owner part in ds, carry parts at dsOff of each slot
+  SgParams q = g.p;
+  q.out = ds; q.ldOut = (size_t)ldDs; q.carry = pl->carry ? pl->carry + g.dsOff : nullptr; q.ldC = pl->carryLd;
+  q.Q = 2u * (uint32_t)heads;
+  return gat_ds_fixup(q, st);
+}
+
+extern "C" size_t roc_gat_finish_workspace_bytes(int H) { return (size_t)GAT_FINISH_BLOCKS * 2 * (size_t)H * sizeof(float); }
+
+extern "C" int roc_gat_bwd_finish(int64_t rows, int H, int heads, const float* h, int64_t ldH, const float* attW,
+                                  const float* ds, int64_t ldDs, float* inGrad, int64_t ldIn, float* attGrad,
+                                  void* workspace, size_t workspaceBytes, roc_stream_t stream) {
+  if (rows < 0 || !h || !attW || !ds || !inGrad || !attGrad || !workspace || ldH < H || ldIn < H || ldDs < 2 * heads)
+    return ROC_ERR_INVALID;
+  if (!gat_shape_ok(H, heads)) return ROC_ERR_UNSUPPORTED;
+  if (workspaceBytes < roc_gat_finish_workspace_bytes(H)) return ROC_ERR_INVALID;
+  cudaStream_t st = as_stream(stream);
+  float* part = static_cast<float*>(workspace);
+  const uint32_t nb = rows > 0 ? (uint32_t)std::min<int64_t>(GAT_FINISH_BLOCKS, (rows + 63) / 64) : 1u;
+  k_gat_finish<<<nb, GAT_FINISH_THREADS, 0, st>>>(rows, H, H / heads, heads, h, ldH, attW, ds, ldDs, inGrad, ldIn, part);
+  ROC_LAUNCH_CHECK();
+  k_gat_da_reduce<<<(2 * H + 255) / 256, 256, 0, st>>>(H, nb, part, attGrad);
+  ROC_LAUNCH_CHECK();
+  return ROC_OK;
 }

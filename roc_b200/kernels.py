@@ -96,6 +96,36 @@ class SgPlan:
                                       _ptr(out), _ld(out), _stream()), "roc_sg_arg_backward")
         return out
 
+    # ---- graph attention (roc_gat_* in include/roc_b200.h).  Tensors the gathers index (h, att, bst, dOut) hold
+    # the plan's own rows first: row r of them is local row r, further rows are what col ids beyond nloc name.
+    def gat_reserve(self, h, heads):
+        check(lib.roc_gat_plan_reserve(self.handle, int(h), int(heads)), "roc_gat_plan_reserve")
+
+    def gat_forward(self, x, att, heads, slope=0.2, out=None, bst=None):
+        """Returns (out [nloc][H], bst [rows of att][round_up4(2K)] with lse of the own rows in columns 0..K-1)."""
+        nloc = self.row_right - self.row_left + 1
+        h = x.shape[1]
+        if out is None:
+            out = padded(nloc, h, x.device) if _ld(x) % 4 == 0 else torch.empty((nloc, h), device=x.device)
+        if bst is None:
+            bst = padded(att.shape[0], 2 * heads, x.device)
+        check(lib.roc_gat_forward(self.handle, h, heads, float(slope), _ptr(x), _ld(x), _ptr(att), _ld(att), _ptr(bst),
+                                  _ld(bst), _ptr(out), _ld(out), _stream()), "roc_gat_forward")
+        return out, bst
+
+    def gat_backward(self, x, att, bst, gy, heads, slope=0.2, dx=None, ds=None):
+        """The backward gather: returns (dh_agg [nloc][H], ds [nloc][round_up4(2K)] = ds_src | ds_dst)."""
+        nloc = self.row_right - self.row_left + 1
+        h = x.shape[1]
+        if dx is None:
+            dx = padded(nloc, h, x.device) if _ld(x) % 4 == 0 else torch.empty((nloc, h), device=x.device)
+        if ds is None:
+            ds = padded(nloc, 2 * heads, x.device)
+        check(lib.roc_gat_backward(self.handle, h, heads, float(slope), _ptr(x), _ld(x), _ptr(att), _ld(att),
+                                   _ptr(bst), _ld(bst), _ptr(gy), _ld(gy), _ptr(dx), _ld(dx), _ptr(ds), _ld(ds),
+                                   _stream()), "roc_gat_backward")
+        return dx, ds
+
     def close(self):
         if self.handle:
             lib.roc_sg_plan_destroy(self.handle)
@@ -299,3 +329,32 @@ def adam_update(w, g, m, v, alpha_t, beta1, beta2, wd, eps):
 
 def launch_count():
     return lib.roc_launch_count()
+
+
+# ---- graph attention, per-node kernels
+def gat_scores(x, att_w, heads, rows=None):
+    """att[r] = (s_src[r][0..K) | s_dst[r][0..K)) for rows 0 .. rows-1 (default: all of x), [x rows][round_up4(2K)];
+    att_w: the [2][H] parameter (row 0 a_src, row 1 a_dst)."""
+    rows = x.shape[0] if rows is None else rows
+    att = padded(x.shape[0], 2 * heads, x.device)
+    check(lib.roc_gat_scores(rows, x.shape[1], heads, _ptr(x), _ld(x), _ptr(att_w), _ptr(att), _ld(att), _stream()),
+          "roc_gat_scores")
+    return att
+
+
+def gat_c(gy, out, bst, heads):
+    """c = <gy, out> per row and head into bst's columns K..2K-1 (rows of gy)."""
+    check(lib.roc_gat_bwd_c(gy.shape[0], gy.shape[1], heads, _ptr(gy), _ld(gy), _ptr(out), _ld(out), _ptr(bst),
+                            _ld(bst), _stream()), "roc_gat_bwd_c")
+    return bst
+
+
+def gat_finish(x, att_w, ds, dx, heads):
+    """dx[r] += ds_src[r] a_src + ds_dst[r] a_dst per head, in place, for the rows of dx; returns da [2][H]."""
+    h = x.shape[1]
+    da = torch.empty((2, h), device=x.device)
+    nbytes = lib.roc_gat_finish_workspace_bytes(h)
+    ws = torch.empty(nbytes // 4, device=x.device)
+    check(lib.roc_gat_bwd_finish(dx.shape[0], h, heads, _ptr(x), _ld(x), _ptr(att_w), _ptr(ds), _ld(ds), _ptr(dx),
+                                 _ld(dx), _ptr(da), _ptr(ws), nbytes, _stream()), "roc_gat_bwd_finish")
+    return da

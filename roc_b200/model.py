@@ -76,6 +76,7 @@ class Model:
     def __init__(self, host, seed=None):
         self.host = host
         self.h = host.h
+        self._gat_heads = {}
         if seed is not None:
             lib.roc_host_srand(seed)     # std::srand(config.seed), gnn.cc:56
 
@@ -104,6 +105,27 @@ class Model:
         out = np.empty((rows, hidden), dtype=np.uint32)
         check(lib.roc_host_sg_arg(self.h, t, out.ctypes.data), "roc_host_sg_arg")
         return out
+
+    def graph_attention(self, t, heads=1, negative_slope=0.2):
+        """GAT over tensor t (width H = heads * F, heads concatenated); owns a [2][H] parameter (a_src, a_dst)."""
+        out = lib.roc_host_graph_attention(self.h, t, int(heads), float(negative_slope))
+        self._gat_heads[out] = int(heads)
+        return out
+
+    def gat_lse(self, t):
+        """lse [rows][heads] of the graph_attention whose output is `t`, own rows, as the latest forward left it."""
+        rows, _, _ = self.tensor_shape(t)
+        out = np.empty((rows, self._gat_heads[t]), dtype=np.float32)
+        check(lib.roc_host_gat_lse(self.h, t, out.ctypes.data), "roc_host_gat_lse")
+        return out
+
+    def gat_param(self, t):
+        """Parameter index of the [2][H] attention weight (row 0 a_src, row 1 a_dst) of the graph_attention whose
+        output is `t`."""
+        p = lib.roc_host_gat_param(self.h, t)
+        if p < 0:
+            raise _lib.RocError("tensor %d is not the output of a graph_attention" % t)
+        return p
 
     def relu(self, t):
         return lib.roc_host_relu(self.h, t)
@@ -320,3 +342,33 @@ def build_sage(model, layers, dropout_rate, aggr="mean", lr=0.01, weight_decay=0
     model.adam(lr, weight_decay)
     model.init()
     return {"input": x, "label": label, "mask": mask, "logits": t, "relu_outs": relu_outs, "sage_outs": sage_outs}
+
+
+def build_gat(model, layers, heads, dropout_rate, negative_slope=0.2, lr=0.01, weight_decay=0.05):
+    """Graph attention network (Velickovic et al. 2018) for `layers` = [in, h_1, ..., out]:
+
+        t  = graph_attention(linear(dropout(t), layers[i]), K_i)     # K_i = heads, 1 in the last layer
+        t  = relu(t)                                                  # all but the last layer
+
+    Each hidden width layers[i] is K_i heads of layers[i] / K_i features, concatenated.  "gat_outs" are the
+    attention outputs (Model.gat_lse / gat_param take them), "att_params" the parameter indices of their [2][H]
+    attention weights."""
+    L = len(layers)
+    x = model.create_node_tensor(layers[0])
+    label = model.create_node_tensor(layers[-1])
+    mask = model.create_node_tensor(1, is_int=True)
+    t = x
+    relu_outs, gat_outs = [], []
+    for i in range(1, L):
+        d = model.dropout(t, dropout_rate)
+        t = model.linear(d, layers[i], _lib.AC_MODE_NONE)
+        t = model.graph_attention(t, heads if i != L - 1 else 1, negative_slope)
+        gat_outs.append(t)
+        if i != L - 1:
+            t = model.relu(t)
+            relu_outs.append(t)
+    model.softmax_cross_entropy(t, label, mask)
+    model.adam(lr, weight_decay)
+    model.init()
+    return {"input": x, "label": label, "mask": mask, "logits": t, "relu_outs": relu_outs, "gat_outs": gat_outs,
+            "att_params": [model.gat_param(g) for g in gat_outs]}
